@@ -21,6 +21,12 @@ value, end-to-end value and a parity spot-check against the oracle made inside t
 
 `--impl reference` times the reference path's CPU restatement (oracle/; the reference cannot be built as a whole,
 SURVEY.md F3) with all host threads on the same workload and prints the same JSON line.
+
+`--dump-outputs DIR` writes what the headline's device-resident path returned in its last timed step for a fixed,
+seeded sample of the batch (dump_outputs below), so that two builds can be compared output for output on identical
+inputs.  `--steps` sets the headline's timed steps (device-resident and end to end); the other workloads time fixed
+counts.  bench.py runs the libraries build() left in the tree, stops if libswm_orb.so is older than its sources, and
+writes nothing in the tree.
 """
 import argparse
 import ctypes as C
@@ -338,6 +344,7 @@ class ExtractBench:
         self.wptrs = [C.c_void_p(ws.cuda_stream) for ws in self.wstreams]
         self.KP = KP_DTYPE
         self.nfeat = nfeat
+        self.launches = 0
 
     def step_device(self):
         """One pass over the B resident frames: chunks of `hb` frames round-robin over the handles / streams, as
@@ -347,9 +354,7 @@ class ExtractBench:
             i, f0 = c % self.nh, c * hb
             self.dex[i].extract_batch_device(self.d_img[f0:].data_ptr(), hb, w, h, w, w * h, self.d_kps[f0:].data_ptr(),
                                              self.d_desc[f0:].data_ptr(), self.cap, self.d_n[f0:].data_ptr(), self.wptrs[i])
-
-    def launches_per_step(self):
-        return (self.B // self.hb) * self.dex[0].last_launches()
+            self.launches += self.dex[i].last_launches()
 
     def time_device(self, steps, warmup):
         torch, ctx = self.ctx.torch, self.ctx
@@ -360,6 +365,7 @@ class ExtractBench:
         e0.record(ctx.stream)
         for ws in self.wstreams:
             ws.wait_event(e0)
+        self.launches = 0   # kernels launched by the timed steps
         for _ in range(steps):
             self.step_device()
         for ws in self.wstreams:
@@ -414,6 +420,42 @@ class ExtractBench:
 
     def bytes_per_frame(self):
         return self.w * self.h, self.cap * (28 + 32) + 4
+
+
+def headline_frames(batch, rank=0):
+    """The headline's distinct synthetic frames (at most 512, tiled to the batch: inputs >> L2); frame i of the batch
+    is frames[i % len(frames)]."""
+    from swarmmap_b200 import synth
+    return synth.make_batch(min(batch, 512), W, H, 20220410 + rank)
+
+
+DUMP_FRAMES = 256    # x at most ~1030 keypoints x (7 + 32) float32 per frame: about 41 MB
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(eb, out_dir):
+    """Writes the device-resident path's outputs of its last timed step for a fixed, seeded sample of DUMP_FRAMES
+    frames of the batch (every frame when the batch is smaller), as float32 arrays:
+      frames.npy       (S,)        batch indices of the sample, ascending
+      n_keypoints.npy  (S,)        keypoints per frame
+      keypoints.npy    (sum n, 7)  x, y, size, angle, response, octave, class_id (KP_DTYPE order; the integers are exact)
+      descriptors.npy  (sum n, 32) descriptor bytes
+    Keypoints and descriptors are the frames' valid rows, concatenated in sample order."""
+    torch = eb.ctx.torch
+    idx = np.sort(np.random.default_rng(0).choice(eb.B, min(eb.B, DUMP_FRAMES), replace=False))
+    sel = torch.from_numpy(idx).to(eb.ctx.dev)
+    n = eb.d_n[sel].cpu().numpy()
+    m = max(int(n.max()), 1)
+    kps = eb.d_kps[sel, :m].cpu().numpy().view(eb.KP).reshape(len(idx), m)
+    desc = eb.d_desc[sel, :m].cpu().numpy()
+    kp = np.concatenate([k[:c] for k, c in zip(kps, n)])
+    out = {"frames": idx.astype(np.float32), "n_keypoints": n.astype(np.float32),
+           "keypoints": np.stack([kp[f].astype(np.float32) for f in eb.KP.names], 1),
+           "descriptors": np.concatenate([d[:c] for d, c in zip(desc, n)]).astype(np.float32)}
+    assert sum(a.nbytes for a in out.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------- config 2
@@ -889,20 +931,28 @@ def workload_place(ctx, cpu):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline, device-resident and end to end (the other workloads time fixed counts)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batch", type=int, default=8192, help="frames per step per GPU (8192 x 20 steps = a timed region above 1 s)")
     ap.add_argument("--impl", default="swm", choices=["swm", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only", default="", help="comma list of workloads to run besides the headline (kitti,tracking,place); default all")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the headline's outputs of its last timed step (rank 0, sampled frames) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "swm":
+        ap.error("--dump-outputs writes the outputs of --impl swm")
     args.warmup = max(args.warmup, 3) if args.impl == "swm" else args.warmup
     if args.impl == "reference":
         run_reference(args)
         return
 
     from swarmmap_b200 import build, synth
-    build.build()
+    if build.needs_build():
+        raise SystemExit(f"{build.LIB} is missing or older than its sources: rebuild it (python -m swarmmap_b200.build)")
     from swarmmap_b200 import _lib
     from swarmmap_b200.orb import ORBextractor
     ctx = Ctx(args)
@@ -911,14 +961,16 @@ def main():
     cpu = not args.no_cpu_baseline
     only = set(x for x in args.only.split(",") if x) or {"kitti", "tracking", "place"}
 
-    # ---- headline: extraction of B frames per step (512 distinct synthetic frames, tiled to B; inputs >> L2)
-    distinct = min(B, 512)
-    frames = synth.make_batch(distinct, W, H, 20220410 + rank)
+    # ---- headline: extraction of B frames per step
+    frames = headline_frames(B, rank)
+    distinct = len(frames)
     eb = ExtractBench(ctx, frames, NFEAT, B, handle_batch=256, nh=4)  # 256-frame calls round-robin over 4 handles / streams (64-frame calls: 151 k instead of 158 k frames/s)
     sampler = ClockSampler(ctx.local_rank)
     sampler.start()
     ms_total, n_kp = eb.time_device(args.steps, args.warmup)
-    launches = eb.launches_per_step() * args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eb, args.dump_outputs)
+    launches = eb.launches
     eb.setup_e2e(8, 64)
     ms_e2e, kp_e2e = eb.time_e2e(args.steps, args.warmup)
     assert kp_e2e == n_kp * args.steps, (kp_e2e, n_kp, args.steps)  # the streamed path produced the same keypoints

@@ -40,7 +40,8 @@ def _p(a):
 @pytest.fixture(scope="module")
 def refc():
     if not os.path.exists(LIB):
-        pytest.skip("oracle/_ref/libref_cuda.so not built (make -C oracle ref, needs /root/reference)")
+        pytest.skip("needs oracle/_ref/libref_cuda.so, compiled by `make -C oracle ref` "
+                    "from the reference project's sources, which the repository does not contain")
     L = C.CDLL(LIB)
     assert L.refc_device_ok()
     L.refc_fast_score_map.restype = None
@@ -53,7 +54,8 @@ def refc():
 def ref_tables():
     """umax and the rBRIEF pattern as the reference's own ORBextractor constructor hands them to the GPU."""
     if not os.path.exists(XLIB):
-        pytest.skip("oracle/_ref/liborbextractor_ref.so not built")
+        pytest.skip("needs oracle/_ref/liborbextractor_ref.so, compiled by `make -C oracle ref` "
+                    "from the reference project's sources, which the repository does not contain")
     X = C.CDLL(XLIB)
     X.ref_orb_create.restype = C.c_void_p
     X.ref_orb_create.argtypes = [C.c_int, C.c_float, C.c_int, C.c_int, C.c_int]

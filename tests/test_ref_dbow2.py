@@ -14,7 +14,8 @@ from swarmmap_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "oracle", "_ref", "libdbow2_ref.so")
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason="oracle/_ref/libdbow2_ref.so not built (make -C oracle ref)")
+pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason="needs oracle/_ref/libdbow2_ref.so, compiled by `make -C oracle ref` "
+                                                                "from the reference project's sources, which the repository does not contain")
 
 
 @pytest.fixture(scope="module")

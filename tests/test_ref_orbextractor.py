@@ -17,7 +17,8 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "oracle", "_ref", "liborbextractor_ref.so")
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason="oracle/_ref/liborbextractor_ref.so not built (make -C oracle ref)")
+pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason="needs oracle/_ref/liborbextractor_ref.so, compiled by `make -C oracle ref` "
+                                                                "from the reference project's sources, which the repository does not contain")
 
 
 def _p(a):

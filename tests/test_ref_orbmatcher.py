@@ -13,7 +13,8 @@ import ref_matcher_lib as R
 from swarmmap_b200 import synth
 from swarmmap_b200.matcher import FeatureVector, Frame
 
-pytestmark = pytest.mark.skipif(not R.available(), reason="oracle/_ref/liborbmatcher_ref.so not built (make -C oracle ref)")
+pytestmark = pytest.mark.skipif(not R.available(), reason="needs oracle/_ref/liborbmatcher_ref.so, compiled by `make -C oracle ref` "
+                                                          "from the reference project's sources, which the repository does not contain")
 
 W, H = 640, 400
 K = R.EUROC_K

@@ -9,7 +9,8 @@ from swarmmap_b200 import synth
 import oracle_lib
 import ref_matcher_lib
 
-pytestmark = pytest.mark.skipif(not ref_matcher_lib.available(), reason="oracle/_ref/liborbmatcher_ref.so not built")
+pytestmark = pytest.mark.skipif(not ref_matcher_lib.available(), reason="needs oracle/_ref/liborbmatcher_ref.so, compiled by `make -C oracle ref` "
+                                                                        "from the reference project's sources, which the repository does not contain")
 
 
 def _views(w, h, nfeat, seed, **kw):
