@@ -7,6 +7,7 @@ import os
 import numpy as np
 import pytest
 
+import orb_ref
 from swarmmap_b200 import synth
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -150,6 +151,7 @@ def test_gpu_reproduces_extract_golden(swm, name):
         assert sha(ex.debug_plane(0, l, 0)) == str(g[f"plane_sha_{l}"])
         assert sha(ex.debug_plane(0, l, 1)) == str(g[f"blur_sha_{l}"])
         assert min(len(ex.debug_points(0, l, 0)), 10000) == int(g[f"fast_count_{l}"])
+    orb_ref.check_extractor_frame(ex, 0, kps, desc, score=False, what=name)
 
 
 @pytest.mark.gpu

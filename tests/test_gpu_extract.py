@@ -1,11 +1,14 @@
 """GPU parity of the extractor against the CPU oracle, stage by stage (run with -m gpu on a B200).
 
 Bar (BASELINE.json north_star): pyramid, FAST keypoint set, quadtree selection bit-exact;
-orientation within 1e-4 rad; >= 99.9 % of descriptor bits identical.
+orientation within 1e-4 rad; >= 99.9 % of descriptor bits identical.  On top of that bar every keypoint the GPU
+returns is checked on its own against the float64 reference of tests/orb_ref.py (coordinates, size, response,
+angle within 4e-6 rad, no descriptor bit that float32 rounding cannot explain).
 """
 import numpy as np
 import pytest
 
+import orb_ref
 from swarmmap_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -24,7 +27,7 @@ def _extractors(oracle, nfeatures, max_batch=1, **kw):
 def _check_frame(gpu, cpu, img, frame=0, kd=None):
     """Compares every intermediate of `frame` of the last GPU batch with the oracle run on img."""
     okps, odesc = cpu(img)
-    for l in range(8):
+    for l in range(gpu.GetLevels()):
         np.testing.assert_array_equal(gpu.debug_plane(frame, l, 0), cpu.level(l, 0), err_msg=f"bordered plane L{l}")
         np.testing.assert_array_equal(gpu.debug_plane(frame, l, 2), cpu.level(l, 2), err_msg=f"FAST score map L{l}")
         np.testing.assert_array_equal(gpu.debug_plane(frame, l, 1), cpu.level(l, 1), err_msg=f"blurred plane L{l}")
@@ -49,6 +52,9 @@ def _check_frame(gpu, cpu, img, frame=0, kd=None):
         bits = np.unpackbits(desc ^ odesc).sum()
         frac = 1.0 - bits / float(desc.size * 8)
         assert frac >= DESC_BIT_FRACTION, f"descriptor bit agreement {frac}"
+        st = orb_ref.check_extractor_frame(gpu, frame, kps, desc)
+        print(f"float64 reference: {st['n']} keypoints, max angle error {st['max_angle_err_rad']:.2e} rad, "
+              f"{st['ambiguous_bits']} ambiguous bits")
     return okps, odesc
 
 
@@ -104,7 +110,7 @@ def test_batch_matches_single(oracle, swm):
         bits = np.unpackbits(desc[f, :n[f]] ^ odesc).sum()
         assert 1.0 - bits / float(odesc.size * 8) >= DESC_BIT_FRACTION
     # intermediates of the last chunk (frames 4,5 sit in slots 0,1)
-    _check_frame(gpu, cpu, imgs[5], 1)
+    _check_frame(gpu, cpu, imgs[5], 1, (kps[5, :n[5]], desc[5, :n[5]]))
 
 
 def test_bench_batch_size_invariances(oracle, swm):
@@ -144,12 +150,27 @@ def test_bench_batch_size_invariances(oracle, swm):
             np.testing.assert_array_equal(k1[s, :n1[s]][fld], okps[fld])
 
 
-@pytest.mark.parametrize("w,h", [(640, 480), (333, 257), (200, 150), (1001, 301)])
+# the layout limits of 8 levels at 1.2 (oracle.level_sizes): 200x138 has a 39 px coarsest level (the smallest side
+# accepted); 528x140 gives DistributeOctTree round((W - 32) / (H - 32)) == 16 initial nodes on its coarsest level
+# (the largest accepted; the live-node bound there is 4 x 16, not quota + 3); 4000 px is the widest level accepted
+@pytest.mark.parametrize("w,h", [(640, 480), (333, 257), (200, 150), (1001, 301), (200, 138), (528, 140), (3990, 400),
+                                 (4000, 400)])
 def test_odd_sizes(oracle, swm, w, h):
     gpu, cpu = _extractors(oracle, 500)
     img = synth.make_frame(w, h, 1234 + w)
     kps, desc = gpu(img)
     _check_frame(gpu, cpu, img, 0, (kps, desc))
+
+
+# one past each limit: a 38 px coarsest level, 17 initial quadtree nodes, a 4001 px level
+@pytest.mark.parametrize("w,h", [(200, 137), (529, 140), (4001, 400)])
+def test_sizes_past_the_limits_refused(swm, w, h):
+    from swarmmap_b200.orb import ORBextractor, SwmError
+    gpu = ORBextractor(500, 1.2, 8, 20, 7)
+    with pytest.raises(SwmError, match="SWM_E_INVALID"):
+        gpu(synth.make_frame(w, h, 1234 + w))
+    kps, _ = gpu(synth.make_frame(640, 480, 1))  # the handle stays usable
+    assert len(kps) > 400
 
 
 def test_textureless_and_noise(oracle, swm):
@@ -213,6 +234,34 @@ def test_other_extractor_settings(oracle, swm, cfg):
         np.testing.assert_array_equal(kps[fld], okps[fld], err_msg=fld)
     assert 1.0 - np.unpackbits(desc ^ odesc).sum() / float(desc.size * 8) >= DESC_BIT_FRACTION
     np.testing.assert_array_equal(gpu.mnFeaturesPerLevel, oracle.level_quotas(nf, sf, nl))
+
+
+# max per-level quota of nfeatures at 8 levels, 1.2 (oracle.level_quotas): 2359 -> 512, 2360 -> 513, 4717 -> 1024,
+# 4718 -> 1025, 9432 -> 2048 (the largest accepted), i.e. both sides of each quadtree instantiation
+# (ot_max_live(512 / 1024 / 2048)); one level of 2000 takes the 2048 instantiation with a single level
+@pytest.mark.parametrize("cfg", [(2359, 1.2, 8, 20, 7), (2360, 1.2, 8, 20, 7), (4717, 1.2, 8, 20, 7),
+                                 (4718, 1.2, 8, 20, 7), (9432, 1.2, 8, 20, 7), (2000, 1.2, 1, 20, 7)],
+                         ids=["q512", "q513", "q1024", "q1025", "q2048", "q2000-1level"])
+def test_quota_boundaries(oracle, swm, cfg):
+    """White noise at 1241x376 leaves more level-0 FAST candidates than any quota, so the quadtree runs to the quota."""
+    from swarmmap_b200.orb import ORBextractor
+    nf, sf, nl, ini, mn = cfg
+    q = oracle.level_quotas(nf, sf, nl)
+    assert {2359: 512, 2360: 513, 4717: 1024, 4718: 1025, 9432: 2048, 2000: 2000}[nf] == q.max()
+    gpu = ORBextractor(nf, sf, nl, ini, mn, debug_score=True)
+    np.testing.assert_array_equal(gpu.mnFeaturesPerLevel, q)
+    cpu = oracle.Extractor(nf, sf, nl, ini, mn)
+    img = np.random.default_rng(nf).integers(0, 256, (376, 1241), dtype=np.uint8)
+    kps, desc = gpu(img)
+    _check_frame(gpu, cpu, img, 0, (kps, desc))
+    assert (kps["octave"] == 0).sum() >= q[0]
+
+
+def test_quota_past_2048_refused(oracle, swm):
+    from swarmmap_b200.orb import ORBextractor, SwmError
+    assert oracle.level_quotas(9433).max() == 2049
+    with pytest.raises(SwmError, match="SWM_E_INVALID"):
+        ORBextractor(9433, 1.2, 8, 20, 7)
 
 
 def test_size_change_on_one_handle(oracle, swm):

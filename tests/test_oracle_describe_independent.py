@@ -2,22 +2,10 @@
 IC_Angle_kernel, code/src/cuda/Orb_gpu.cu:63-104 calcOrb_kernel) against the oracle's orc_extract output, for the
 octave-0 keypoints of a frame (their coordinates are level coordinates).  The un-blurred and blurred level planes the
 stages read are the ones tests/test_oracle_cv2.py pins to cv2."""
-import os
-import re
-
 import numpy as np
 
+from orb_ref import load_pattern
 from swarmmap_b200 import synth
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def load_pattern():
-    txt = open(os.path.join(ROOT, "oracle", "orb_pattern_data.inc")).read()
-    body = txt[txt.index("{") + 1:txt.index("};")]
-    vals = np.array([int(v) for v in re.findall(r"-?\d+", body)], np.int64)
-    assert len(vals) == 1024
-    return vals.reshape(512, 2)  # (x, y) per sample point; bit i compares point 2i with point 2i + 1
 
 
 def test_ic_angle_and_rbrief_vs_numpy(oracle):
