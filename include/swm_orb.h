@@ -28,6 +28,9 @@
  *                               MapPoint::ComputeDistinctiveDescriptors    src/ORBmatcher.cc:599-1221, src/MapPoint.cc:361-391
  *   swm_match_*_batch           the same Search* calls for many agents in one call (src/Tracking.cc:470-472,619-626,715-737)
  *   swm_vocab_*, swm_bow_*      DBoW2 transform (Frame::ComputeBoW)  Thirdparty/DBoW2/DBoW2/TemplatedVocabulary.h:1151-1283
+ *                               and ORBVocabulary::score (L1Scoring::score, ScoringObject.cpp)
+ *   swm_kfdb_*                  KeyFrameDatabase (add / erase / clear / DetectRelocalizationCandidates /
+ *                               DetectLoopCandidates)                src/KeyFrameDatabase.cc
  *   swm_db_*                    role of KeyFrameDatabase::DetectLoopCandidates + SearchByBoW(KF,KF) in
  *                               AgentMediator::CheckOverlapCandidates (src/AgentMediator.cc:140-202), recast as
  *                               brute-force Hamming top-k over a sharded descriptor database (BASELINE config 5);
@@ -421,6 +424,56 @@ int swm_bow_transform(swm_vocab* v, const uint8_t* desc, const int32_t* n, int b
                       const swm_bow_out* out);
 /* The same for one resident frame (cap = swm_frame_size(f)); the descriptors never leave the device. */
 int swm_bow_transform_frame(swm_vocab* v, const swm_frame* f, int levelsup, const swm_bow_out* out);
+/* ORBVocabulary::score (TemplatedVocabulary.h, DBoW2 ScoringObject.cpp L1Scoring::score) of npairs pairs of
+ * BowVectors: out[i] = score(a_i, b_i), bit-exact.  Pair i's vectors are a_words / a_values[a_offsets[i] ..
+ * a_offsets[i+1]) and likewise for b; word ids strictly ascending.  L1_NORM vocabularies only (SWM_E_INVALID
+ * otherwise). */
+int swm_bow_score(swm_vocab* v, int npairs, const int32_t* a_offsets, const uint32_t* a_words, const double* a_values,
+                  const int32_t* b_offsets, const uint32_t* b_words, const double* b_values, double* out);
+
+/* ------------------------------------------------------------------ KeyFrameDatabase (place recognition)
+ * KeyFrameDatabase::{add, erase, clear, DetectRelocalizationCandidates, DetectLoopCandidates} (ORB-SLAM2's
+ * KeyFrameDatabase.cc as SwarmMap carries it; callers Tracking::Relocalization, LoopClosing::DetectLoop,
+ * AgentMediator::CheckOverlapCandidates) on one device, with DBoW2's L1 score.  Results equal the reference's
+ * ordered candidate lists exactly under the definitions of DESIGN.md section 2: stale reloc scores are reproduced
+ * (kept per keyframe id for the database's lifetime, through erase / re-add / clear), they start at 0.0f, and every
+ * query is a fresh query.  A batch of queries equals the same queries issued one after another in array order.
+ *
+ * A query has two phases because the reference reads the covisibility graph only for the scored keyframes:
+ *   swm_kfdb_query   scores the database against nq BowVectors and returns, per query, lScoreAndMatch in list
+ *                    order (keyframe ids and float scores) in the CSR scored_offsets[nq + 1] / scored_ids /
+ *                    scored_scores;
+ *   swm_kfdb_finish  takes each scored entry's GetBestCovisibilityKeyFrames(10) (ids, in order; CSR aligned with the
+ *                    scored entries, ids not in the database are ignored) and returns the candidates per query in
+ *                    the CSR cand_offsets[nq + 1] / cand_ids.
+ * finish without a preceding query, or after an add / erase / clear since it, returns SWM_E_STATE.  A capacity too
+ * small returns SWM_E_CAPACITY with the size needed in scored_offsets[nq] / cand_offsets[nq]; a query that fails
+ * this way changes no state and can be repeated with a larger buffer. */
+#define SWM_KFDB_RELOC 0 /* DetectRelocalizationCandidates(Frame*) */
+#define SWM_KFDB_LOOP 1  /* DetectLoopCandidates(KeyFrame*, minScore) */
+typedef struct swm_kfdb swm_kfdb; /* opaque: the database on the vocabulary's device */
+/* SWM_E_INVALID unless the vocabulary's scoring type is L1_NORM (ORBvoc's). */
+int swm_kfdb_create(swm_vocab* v, swm_kfdb** out);
+void swm_kfdb_destroy(swm_kfdb* db);
+const char* swm_kfdb_last_error(const swm_kfdb* db);
+int64_t swm_kfdb_size(const swm_kfdb* db); /* live keyframes */
+/* n keyframes; keyframe i: id kf_ids[i], BowVector word_ids / values[offsets[i] .. offsets[i+1]) (ascending word
+ * ids).  SWM_E_INVALID (nothing added) for an id that is live already or a word id >= the vocabulary's size. */
+int swm_kfdb_add(swm_kfdb* db, int n, const uint64_t* kf_ids, const int32_t* offsets, const uint32_t* word_ids,
+                 const double* values);
+int swm_kfdb_erase(swm_kfdb* db, int n, const uint64_t* kf_ids); /* ids that are not live are ignored */
+int swm_kfdb_clear(swm_kfdb* db);
+/* mode SWM_KFDB_RELOC or SWM_KFDB_LOOP; nq queries, query q = q_words / q_values[q_offsets[q] .. q_offsets[q+1]).
+ * Loop mode: min_score[nq], and GetConnectedKeyFrames() of query q = conn_ids[conn_offsets[q] .. conn_offsets[q+1])
+ * (conn_offsets NULL: none); both are ignored in reloc mode. */
+int swm_kfdb_query(swm_kfdb* db, int mode, int nq, const int32_t* q_offsets, const uint32_t* q_words,
+                   const double* q_values, const float* min_score, const int32_t* conn_offsets,
+                   const uint64_t* conn_ids, int32_t* scored_offsets, uint64_t* scored_ids, float* scored_scores,
+                   int32_t scored_cap);
+int swm_kfdb_finish(swm_kfdb* db, const int32_t* neigh_offsets, const uint64_t* neigh_ids, int32_t* cand_offsets,
+                    uint64_t* cand_ids, int32_t cand_cap);
+/* Device time of the last query + finish pair, from events around each phase's device work, in ms. */
+float swm_kfdb_last_device_ms(const swm_kfdb* db);
 
 /* ------------------------------------------------------------------ place-recognition shard (config 5) */
 typedef struct swm_db swm_db; /* one GPU's shard of the keyframe-descriptor database */

@@ -150,6 +150,17 @@ SYMBOLS = [
     ("swm_vocab_info", _i, [_vp, _vp, _vp, _vp, _vp]),
     ("swm_bow_transform", _i, [_vp, _vp, _vp, _i, _i, _i, _vp]),
     ("swm_bow_transform_frame", _i, [_vp, _vp, _i, _vp]),
+    ("swm_bow_score", _i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    ("swm_kfdb_create", _i, [_vp, _vp]),
+    ("swm_kfdb_destroy", None, [_vp]),
+    ("swm_kfdb_last_error", C.c_char_p, [_vp]),
+    ("swm_kfdb_size", _i64, [_vp]),
+    ("swm_kfdb_add", _i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    ("swm_kfdb_erase", _i, [_vp, _i, _vp]),
+    ("swm_kfdb_clear", _i, [_vp]),
+    ("swm_kfdb_query", _i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int32]),
+    ("swm_kfdb_finish", _i, [_vp, _vp, _vp, _vp, _vp, C.c_int32]),
+    ("swm_kfdb_last_device_ms", C.c_float, [_vp]),
     ("swm_db_create", _i, [_i, _vp, _i64, C.c_int32, _i64, _vp]),
     ("swm_db_create_device", _i, [_i, _vp, _i64, C.c_int32, _i64, _vp]),
     ("swm_db_destroy", None, [_vp]),

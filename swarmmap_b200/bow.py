@@ -8,7 +8,7 @@ import numpy as np
 from . import _lib
 from ._lib import BowOut, SwmError, ptr
 
-__all__ = ["ORBVocabulary", "BowResult"]
+__all__ = ["ORBVocabulary", "BowResult", "bow_csr"]
 
 
 class BowResult:
@@ -26,6 +26,19 @@ class BowResult:
         fv.offsets = np.ascontiguousarray(self.offsets, np.int32)
         fv.feats = np.ascontiguousarray(self.feats, np.uint32)
         return fv
+
+
+def bow_csr(bows):
+    """A list of BowVectors (BowResult objects or (word_ids, values) pairs) -> (offsets int32, words uint32,
+    values float64)."""
+    pairs = [(b.word_ids, b.values) if hasattr(b, "word_ids") else b for b in bows]
+    off = np.zeros(len(pairs) + 1, np.int32)
+    off[1:] = np.cumsum([len(w) for w, _ in pairs])
+    words = np.ascontiguousarray(np.concatenate([np.asarray(w, np.uint32) for w, _ in pairs]) if pairs else
+                                 np.zeros(0, np.uint32), np.uint32)
+    values = np.ascontiguousarray(np.concatenate([np.asarray(v, np.float64) for _, v in pairs]) if pairs else
+                                  np.zeros(0, np.float64), np.float64)
+    return off, words, values
 
 
 class ORBVocabulary:
@@ -92,6 +105,22 @@ class ORBVocabulary:
             z = np.zeros(0, np.uint32)
             return BowResult(z, np.zeros(0), z, np.zeros(1, np.int32), z)
         return self.transform_batch(desc[None], np.array([len(desc)], np.int32), levelsup)[0]
+
+    def score_pairs(self, a, b):
+        """ORBVocabulary::score (DBoW2 L1Scoring::score) of each pair (a[i], b[i]) of BowVectors: BowResult objects or
+        (word_ids, values) pairs.  L1_NORM vocabularies only.  Returns float64 scores, bit-exact."""
+        if len(a) != len(b):
+            raise ValueError("a and b must hold the same number of BowVectors")
+        ao, aw, av = bow_csr(a)
+        bo, bw, bv = bow_csr(b)
+        out = np.zeros(len(a), np.float64)
+        self._check(self._lib.swm_bow_score(self._h, len(a), ptr(ao), ptr(aw), ptr(av), ptr(bo), ptr(bw), ptr(bv),
+                                            ptr(out)), "swm_bow_score")
+        return out
+
+    def score(self, a, b):
+        """ORBVocabulary::score(a, b) of two BowVectors."""
+        return float(self.score_pairs([a], [b])[0])
 
     def transform_frame(self, frame, levelsup=4):
         """The same for a ResidentFrame: the descriptors stay on the device."""

@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libswm_orb.so")
-SOURCES = ["extract.cu", "match.cu", "bow.cu"]
+SOURCES = ["extract.cu", "match.cu", "bow.cu", "kfdb.cu"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-shared", "-ldl"]
 

@@ -260,11 +260,14 @@ struct swm_vocab {
   Buf desc, child_off, child, word, weight;
   Buf in_desc, in_n, word_of, node_of, w_of;
   Buf o_word_ids, o_values, o_n_words, o_node_ids, o_offsets, o_feats, o_n_nodes;
+  PinnedArena score_arena;  // swm_bow_score: operands in, scores out
+  Buf score_out;
   cudaStream_t stream = nullptr;
   void free_all() {
     for (Buf* b : {&desc, &child_off, &child, &word, &weight, &in_desc, &in_n, &word_of, &node_of, &w_of, &o_word_ids,
-                   &o_values, &o_n_words, &o_node_ids, &o_offsets, &o_feats, &o_n_nodes})
+                   &o_values, &o_n_words, &o_node_ids, &o_offsets, &o_feats, &o_n_nodes, &score_out})
       b->release();
+    score_arena.release();
   }
 };
 
@@ -448,4 +451,51 @@ int swm_bow_transform_frame(swm_vocab* v, const swm_frame* f, int levelsup, cons
   return bow_run(v, fv.desc, v->in_n.as<int32_t>(), 1, fv.n, levelsup, out);
 }
 
+int swm_bow_score(swm_vocab* v, int npairs, const int32_t* a_offsets, const uint32_t* a_words, const double* a_values,
+                  const int32_t* b_offsets, const uint32_t* b_words, const double* b_values, double* out) {
+  if (!v) return SWM_E_INVALID;
+  if (v->scoring != 0) { v->err = "swm_bow_score: the vocabulary's scoring type is not L1_NORM"; return SWM_E_INVALID; }
+  if (npairs < 0 || (npairs > 0 && (!a_offsets || !b_offsets || !out))) { v->err = "bad argument"; return SWM_E_INVALID; }
+  if (npairs == 0) return SWM_OK;
+  for (const int32_t* off : {a_offsets, b_offsets}) {
+    const uint32_t* w = off == a_offsets ? a_words : b_words;
+    if (off[0] != 0) { v->err = "offsets[0] must be 0"; return SWM_E_INVALID; }
+    for (int i = 0; i < npairs; i++) {
+      if (off[i + 1] < off[i]) { v->err = "offsets not non-decreasing"; return SWM_E_INVALID; }
+      for (int j = off[i] + 1; j < off[i + 1]; j++)
+        if (w[j] <= w[j - 1]) { v->err = "word ids not strictly ascending"; return SWM_E_INVALID; }
+    }
+    if (off[npairs] > 0 && (!w || !(off == a_offsets ? a_values : b_values))) { v->err = "bad argument"; return SWM_E_INVALID; }
+  }
+  VCK(v, cudaSetDevice(v->device));
+  const size_t na = (size_t)a_offsets[npairs], nb = (size_t)b_offsets[npairs];
+  const size_t bytes = (na + nb) * 12 + (size_t)(npairs + 1) * 8 + (size_t)npairs * 8 + 2048;
+  VCK(v, v->score_arena.begin(bytes, v->stream));
+  const int32_t* da = v->score_arena.put(a_offsets, npairs + 1);
+  const uint32_t* daw = v->score_arena.put(a_words, na);
+  const double* dav = v->score_arena.put(a_values, na);
+  const int32_t* db = v->score_arena.put(b_offsets, npairs + 1);
+  const uint32_t* dbw = v->score_arena.put(b_words, nb);
+  const double* dbv = v->score_arena.put(b_values, nb);
+  VCK(v, v->score_arena.flush(v->stream));
+  VCK(v, v->score_out.ensure((size_t)npairs * 8));
+  VCK(v, launch_l1_score_pairs(npairs, da, daw, dav, db, dbw, dbv, v->score_out.as<double>(), v->stream));
+  double* h = v->score_arena.put(out, 0);  // device address of the read-back slot; its host twin follows
+  uint8_t* h_host = v->score_arena.h + (reinterpret_cast<uint8_t*>(h) - v->score_arena.d);
+  VCK(v, cudaMemcpyAsync(h_host, v->score_out.p, (size_t)npairs * 8, cudaMemcpyDeviceToHost, v->stream));
+  VCK(v, cudaStreamSynchronize(v->stream));
+  memcpy(out, h_host, (size_t)npairs * 8);
+  return SWM_OK;
+}
+
 }  // extern "C"
+
+namespace swm {
+int vocab_props(const swm_vocab* v, VocabProps* out) {
+  if (!v || !out) return SWM_E_INVALID;
+  out->device = v->device;
+  out->scoring = v->scoring;
+  out->n_words = v->n_words;
+  return SWM_OK;
+}
+}  // namespace swm

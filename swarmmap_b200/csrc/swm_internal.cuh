@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cstring>
 #include <string>
 
 #include "../../include/swm_orb.h"
@@ -65,5 +66,54 @@ struct FrameDeviceView {
   cudaEvent_t ready;  // recorded after the frame's last write
 };
 int frame_device_view(const swm_frame* f, FrameDeviceView* out);
+
+// Vocabulary properties for the keyframe database (kfdb.cu); scoring is DBoW2's ScoringType (0 = L1_NORM).
+struct VocabProps {
+  int device, scoring, n_words;
+};
+int vocab_props(const swm_vocab* v, VocabProps* out);
+
+// Host operands of a call packed into one pinned buffer and sent with one copy; results come back through the
+// same buffer.  Grow-only; growing synchronises `stream` first because earlier copies may still read the buffer.
+struct PinnedArena {
+  uint8_t* h = nullptr;
+  uint8_t* d = nullptr;
+  size_t cap = 0, used = 0;
+  cudaError_t begin(size_t bytes, cudaStream_t stream) {
+    bytes += 4096;
+    used = 0;
+    if (bytes <= cap) return cudaSuccess;
+    cudaError_t e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess) return e;
+    release();
+    const size_t want = bytes + bytes / 2;
+    if ((e = cudaMallocHost(&h, want)) != cudaSuccess) return e;
+    if ((e = cudaMalloc(&d, want)) != cudaSuccess) return e;
+    cap = want;
+    return cudaSuccess;
+  }
+  // copies `bytes` of src into the arena; returns the device address its copy will have after flush()
+  template <class T>
+  T* put(const T* src, size_t count) {
+    const size_t off = (used + 255) & ~(size_t)255, bytes = count * sizeof(T);
+    if (bytes) memcpy(h + off, src, bytes);
+    used = off + bytes;
+    return reinterpret_cast<T*>(d + off);
+  }
+  cudaError_t flush(cudaStream_t stream) {
+    return used ? cudaMemcpyAsync(d, h, used, cudaMemcpyHostToDevice, stream) : cudaSuccess;
+  }
+  void release() {
+    if (h) cudaFreeHost(h);
+    if (d) cudaFree(d);
+    h = d = nullptr;
+    cap = used = 0;
+  }
+};
+
+// DBoW2 L1Scoring::score of npairs pairs (a[i], b[i]) of BowVectors in CSR form, one warp per pair (kfdb.cu).
+cudaError_t launch_l1_score_pairs(int npairs, const int32_t* a_off, const uint32_t* a_words, const double* a_values,
+                                  const int32_t* b_off, const uint32_t* b_words, const double* b_values, double* out,
+                                  cudaStream_t stream);
 
 }  // namespace swm

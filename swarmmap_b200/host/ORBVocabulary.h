@@ -5,8 +5,11 @@
 //                                                     (Frame.cc:445-452), KeyFrame::ComputeBoW (KeyFrame.cc:126-133)
 // The tree walk and the assembly of both containers run on the GPU (swm_bow_transform); BowVector / FeatureVector
 // below have DBoW2's container types (std::map<WordId, WordValue>, std::map<NodeId, std::vector<unsigned>>), so the
-// callers' code (KeyFrameDatabase scoring, SearchByBoW's merge walk) compiles unchanged.  score() and the rest of
-// the vocabulary API stay with DBoW2 (out of scope: SURVEY.md section 8).
+// callers' code (SearchByBoW's merge walk) compiles unchanged.
+//   score(a, b)                                       L1Scoring::score (ScoringObject.cpp), on the GPU (swm_bow_score);
+//                                                     LoopClosing::DetectLoop's minScore; L1_NORM vocabularies only
+// KeyFrameDatabase (KeyFrameDatabase.h) runs on the GPU too.  The rest of the vocabulary API stays with DBoW2
+// (DESIGN.md section 8).
 #pragma once
 #include <cstdio>
 #include <map>
@@ -89,6 +92,17 @@ class ORBVocabulary {
     for (int j = 0; j < nn; j++)
       fv.insert(fv.end(), std::make_pair(node_ids[j], std::vector<unsigned int>(feats.begin() + offsets[j],
                                                                                 feats.begin() + offsets[j + 1])));
+  }
+  double score(const DBoW2::BowVector& a, const DBoW2::BowVector& b) const {
+    std::vector<uint32_t> w;
+    std::vector<double> x;
+    for (const auto& e : a) { w.push_back(e.first); x.push_back(e.second); }
+    for (const auto& e : b) { w.push_back(e.first); x.push_back(e.second); }
+    const int32_t ao[2] = {0, (int32_t)a.size()}, bo[2] = {0, (int32_t)b.size()};
+    double out = 0.0;
+    if (swm_bow_score(v_, 1, ao, w.data(), x.data(), bo, w.data() + a.size(), x.data() + a.size(), &out) != SWM_OK)
+      throw std::runtime_error(std::string("ORBVocabulary::score: ") + swm_vocab_last_error(v_));
+    return out;
   }
   swm_vocab* handle() const { return v_; }
 
