@@ -130,8 +130,12 @@ int swm_orb_last_launches(const swm_orb* h);
  * reference's loop: best descriptor distance in the keypoint's row band (octave +-1, disparity in [-3, bf / b]), 11x11
  * SAD refinement over +-5 px in mvImagePyramid[level] as operator() leaves it (blurred in place), parabola fit, 1.5 * 1.4 * median SAD filter.  bf = mbf
  * (baseline x fx), b = mb (baseline in metres).  cap >= swm_orb_max_keypoints(left), or the cap the batch was extracted
- * with; host outputs, returns after the results are in place. */
-int swm_orb_stereo_match(swm_orb* left, swm_orb* right, float bf, float b, float* u_right, float* depth, int cap);
+ * with.  batch = the number of frame rows u_right and depth hold; it must equal the resident batch: fewer rows return
+ * SWM_E_CAPACITY, more return SWM_E_INVALID (swm_orb_extract_batch keeps only its last chunk of at most
+ * cfg.max_batch frames resident; swm_orb_extract and the C++ operator() leave one frame).  Slots past the frame's
+ * keypoint count are unspecified.  Host outputs, returns after the results are in place. */
+int swm_orb_stereo_match(swm_orb* left, swm_orb* right, float bf, float b, float* u_right, float* depth, int cap,
+                         int batch);
 /* Re-runs the selected stages on the data of the last *_device/_batch call (the caller brackets it with
  * CUDA events on `stream`): per-stage timing for bench.py's roofline and stage breakdown. */
 int swm_orb_run_stage(swm_orb* h, int stage_mask, int batch, void* stream);

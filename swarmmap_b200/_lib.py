@@ -106,7 +106,7 @@ SYMBOLS = [
     ("swm_orb_max_keypoints", _i, [_vp]),
     ("swm_orb_last_launches", _i, [_vp]),
     ("swm_orb_run_stage", _i, [_vp, _i, _i, _vp]),
-    ("swm_orb_stereo_match", _i, [_vp, _vp, C.c_float, C.c_float, _vp, _vp, _i]),
+    ("swm_orb_stereo_match", _i, [_vp, _vp, C.c_float, C.c_float, _vp, _vp, _i, _i]),
     ("swm_orb_set_debug", _i, [_vp, _i]),
     ("swm_orb_debug_plane", _i, [_vp, _i, _i, _i, _vp, _i]),
     ("swm_orb_debug_points", _i, [_vp, _i, _i, _i, _vp, _i]),

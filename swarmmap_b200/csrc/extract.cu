@@ -981,10 +981,11 @@ int swm_orb_extract(swm_orb* h, const uint8_t* img, int w, int h_px, int stride,
   return rc;
 }
 
-int swm_orb_stereo_match(swm_orb* left, swm_orb* right, float bf, float b, float* u_right, float* depth, int cap) {
+int swm_orb_stereo_match(swm_orb* left, swm_orb* right, float bf, float b, float* u_right, float* depth, int cap,
+                         int batch) {
   if (!left || !right) return SWM_E_INVALID;
   swm_orb* h = left;
-  if (!u_right || !depth || !(bf > 0) || !(b > 0)) { h->err = "bad argument"; return SWM_E_INVALID; }
+  if (!u_right || !depth || !(bf > 0) || !(b > 0) || batch < 1) { h->err = "bad argument"; return SWM_E_INVALID; }
   if (!left->last_kps || !right->last_kps || left->last_batch < 1) { h->err = "both extractors must hold an extracted batch"; return SWM_E_STATE; }
   if (left->device != right->device || left->last_batch != right->last_batch || left->lay.w != right->lay.w ||
       left->lay.h != right->lay.h || left->cfg.nlevels != right->cfg.nlevels || left->cfg.scale_factor != right->cfg.scale_factor) {
@@ -994,6 +995,17 @@ int swm_orb_stereo_match(swm_orb* left, swm_orb* right, float bf, float b, float
   if (left->last_cap >= 65536 || right->last_cap >= 65536) { h->err = "more than 65535 keypoints per frame"; return SWM_E_CAPACITY; }
   const int B = left->last_batch, capl = left->last_cap;
   if (cap < capl) { h->err = "output capacity below the extractor's keypoint capacity"; return SWM_E_CAPACITY; }
+  // The outputs hold `batch` rows and the results cover the resident batch: swm_orb_extract_batch splits a call into
+  // chunks of cfg.max_batch frames and only the last chunk stays resident, so more rows than that cannot be filled.
+  if (batch < B) {
+    h->err = "output rows (" + std::to_string(batch) + ") below the extracted batch of " + std::to_string(B) + " frames";
+    return SWM_E_CAPACITY;
+  }
+  if (batch > B) {
+    h->err = "batch " + std::to_string(batch) + " exceeds the extracted batch of " + std::to_string(B) +
+             " frames (only the last chunk of at most max_batch frames of an extract call stays resident)";
+    return SWM_E_INVALID;
+  }
   SWM_CK(h, cudaSetDevice(h->device));
   const size_t need = (size_t)B * capl;
   if (need > h->stereo_cap) {

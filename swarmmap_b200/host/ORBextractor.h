@@ -124,7 +124,7 @@ class ORBextractor {
     const int cap = swm_orb_max_keypoints(h_);
     stereo_u_.resize(cap);
     stereo_z_.resize(cap);
-    if (swm_orb_stereo_match(h_, right.h_, mbf, mb, stereo_u_.data(), stereo_z_.data(), cap) != SWM_OK)
+    if (swm_orb_stereo_match(h_, right.h_, mbf, mb, stereo_u_.data(), stereo_z_.data(), cap, 1) != SWM_OK)
       throw std::runtime_error(std::string("ORBextractor::ComputeStereoMatches: ") + swm_last_error(h_));
     if (N > cap) N = cap;
     mvuRight.assign(stereo_u_.begin(), stereo_u_.begin() + N);

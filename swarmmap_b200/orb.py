@@ -132,11 +132,12 @@ class ORBextractor:
 
     def stereo_match(self, right, bf, b, batch):
         """Frame::ComputeStereoMatches (reference Frame.cc:516-690) for the batch this extractor (left view) and `right`
-        (right view) extracted last: returns (mvuRight, mvDepth) as (batch, cap) float32 arrays, -1 = no match."""
+        (right view) extracted last: returns (mvuRight, mvDepth) as (batch, cap) float32 arrays, -1 = no match.
+        `batch` must be the number of frames resident: extract_batch keeps only its last chunk of max_batch frames."""
         cap = self.max_keypoints()
         u = np.empty((batch, cap), np.float32)
         z = np.empty((batch, cap), np.float32)
-        check(self._lib.swm_orb_stereo_match(self._h, right._h, bf, b, ptr(u), ptr(z), cap), self._h,
+        check(self._lib.swm_orb_stereo_match(self._h, right._h, bf, b, ptr(u), ptr(z), cap, batch), self._h,
               "swm_orb_stereo_match")
         return u, z
 

@@ -1,11 +1,13 @@
 """Frame::ComputeStereoMatches on the GPU (swm_orb_stereo_match, csrc/stereo.cuh) against the oracle
-(orc_stereo_matches, itself pinned to the reference's own body in tests/test_ref_stereo.py).  The oracle is fed the
+(orc_stereo_matches, itself pinned to the reference's own body in tests/test_ref_stereo.py) and against the second
+reading of tests/stereo_ref.py.  The oracle is fed the
 GPU extractor's own keypoints, descriptors and pyramid (blurred in place inside its un-blurred border), so the comparison isolates the stereo stage:
 mvuRight and mvDepth must be bit-identical floats."""
 import numpy as np
 import pytest
 
 from swarmmap_b200 import synth
+import stereo_ref
 
 pytestmark = pytest.mark.gpu
 
@@ -31,6 +33,7 @@ def _pairs(w, h, seeds, **kw):
     (752, 480, 1000, {"d_near": 9.0, "d_far": 0.0}, 47.90639384423901, 458.654),
     (640, 400, 1500, {"right_shift": 6}, 40.0, 400.0),
     (1241, 376, 2000, {"d_near": 70.0, "d_far": 2.0}, 386.1448, 718.856),
+    (752, 480, 800, {"d_near": 30.0, "d_far": 25.0}, 47.9, 2000.0),   # maxD = 2000 > image width: wide search band
 ])
 def test_stereo_matches_equal_oracle(oracle, swm, w, h, nfeat, kw, mbf, fx):
     from swarmmap_b200.orb import ORBextractor
@@ -50,6 +53,11 @@ def test_stereo_matches_equal_oracle(oracle, swm, w, h, nfeat, kw, mbf, fx):
         u0, z0, n0 = oracle.stereo_matches(kl[f, :nl[f]], dl[f, :nl[f]], kr[f, :nr[f]], dr[f, :nr[f]], pl, pr, sf, inv_sf, mbf, mb)
         np.testing.assert_array_equal(u[f, :nl[f]].view(np.uint32), u0.view(np.uint32), err_msg=f"mvuRight frame {f}")
         np.testing.assert_array_equal(z[f, :nl[f]].view(np.uint32), z0.view(np.uint32), err_msg=f"mvDepth frame {f}")
+        u1, z1, n1, _ = stereo_ref.stereo_matches(kl[f, :nl[f]], dl[f, :nl[f]], kr[f, :nr[f]], dr[f, :nr[f]], pl, pr, sf,
+                                                  inv_sf, mbf, mb)
+        np.testing.assert_array_equal(u[f, :nl[f]].view(np.uint32), u1.view(np.uint32), err_msg=f"reading frame {f}")
+        np.testing.assert_array_equal(z[f, :nl[f]].view(np.uint32), z1.view(np.uint32), err_msg=f"reading frame {f}")
+        assert n1 == n0
         total += n0
     assert total > 100 * B
 
