@@ -394,6 +394,91 @@ float swm_matcher_last_device_ms(const swm_matcher* m);
 int swm_frames_from_extractor(swm_frame** frames, int count, swm_orb* h, const int32_t* indices, const swm_camera* cam,
                               const float* bounds4);
 
+/* ------------------------------------------------------------------ resident MapPoints and tracking projections
+ * Tracking::SearchLocalPoints (code/src/Tracking.cc:964-1006: the mnLastFrameSeen stamp, Frame::isInFrustum
+ * code/src/Frame.cc:316-375 with MapPoint::PredictScale code/src/MapPoint.cc:476-485, then SearchByProjection(F,
+ * vpMapPoints, th) code/src/ORBmatcher.cc:44-121) and SearchByProjection(cur, last, th, bMono = true)
+ * (ORBmatcher.cc:1223-1354) on the device, from a table of MapPoints that stays resident between frames: a call
+ * uploads the pose and row indices only.  Results equal the swm_match_window forms fed with the reference's projection
+ * (numerics of DESIGN.md section 2).  Stereo branches are not served.
+ *
+ * The table holds per row: world position, normal, mfMinDistance, mfMaxDistance, descriptor, Observations() > 0 and
+ * the bad flag.  Ordering between a table's writers and readers, whatever streams or threads issue them:
+ *   - an upsert waits for the last call that read the table (a write never overtakes a query that still reads it);
+ *   - a query waits for the last upsert of every table it reads. */
+typedef struct swm_mappoints swm_mappoints; /* opaque: the table on one device */
+int swm_mappoints_create(int device, int capacity, swm_mappoints** out);
+void swm_mappoints_destroy(swm_mappoints* t);
+const char* swm_mappoints_last_error(const swm_mappoints* t);
+/* Rows the table holds: 1 + the largest row ever written. */
+int32_t swm_mappoints_size(const swm_mappoints* t);
+/* n rows in one packed upload and one scatter kernel: pos / normal n x 3 floats, min_d / max_d n floats
+ * (mfMinDistance / mfMaxDistance, before the 0.8 / 1.2 factors), desc n x 32 bytes, has_obs / bad n bytes.  A row given
+ * twice takes its last entry.  Capacity grows as needed and keeps the contents; a row never written reads as all zero,
+ * bad, without observations.  Any row < 0 returns SWM_E_INVALID before any device work.  The last-frame projection
+ * projects a row whatever its bad flag (ORBmatcher.cc:1247-1250 does not test isBad()), so a row may only be given to
+ * another MapPoint once no frame refers to the old one. */
+int swm_mappoints_upsert(swm_mappoints* t, int n, const int32_t* rows, const float* pos, const float* normal,
+                         const float* min_d, const float* max_d, const uint8_t* desc, const uint8_t* has_obs,
+                         const uint8_t* bad);
+/* PredictScale's level is the number of thresholds[0 .. nlevels-2] that ratio = mfMaxDistance / dist exceeds
+ * (thresholds[k] = the largest float ratio of level <= k under ceil(logf(ratio) / log_scale_factor) clamped to
+ * [0, nlevels - 1]).  Host only; the projection calls compute these themselves. */
+int swm_predict_scale_thresholds(float log_scale_factor, int32_t nlevels, float* thresholds);
+
+typedef struct swm_projection {
+  float Tcw[12];               /* mTcw rows 0..2, row-major: [Rcw | tcw] */
+  float fx, fy, cx, cy;        /* Frame::fx .. cy; the image bounds are the resident target frame's */
+  const float* scale_factors;  /* mvScaleFactors (nlevels) */
+  float log_scale_factor;      /* mfLogScaleFactor */
+  int32_t nlevels;             /* mnScaleLevels, <= SWM_MAX_LEVELS */
+} swm_projection;
+/* The tracking fields isInFrustum leaves in each MapPoint of the list (mbTrackInView, mTrackProjX / Y, mTrackViewCos,
+ * mnTrackScaleLevel); n_rows entries each, every pointer may be NULL.  0 where not in view. */
+typedef struct swm_track_out {
+  uint8_t* in_view;
+  float* u;
+  float* v;
+  float* view_cos;
+  int32_t* level;
+} swm_track_out;
+
+#define SWM_LOCALMAP_POINTS 0 /* SearchLocalPoints */
+#define SWM_LOCALMAP_LAST 1   /* SearchByProjection(cur, last, th, true) */
+typedef struct swm_localmap_job {
+  int32_t mode;
+  const swm_frame* tgt;         /* the current frame */
+  swm_mappoints* table;
+  const swm_projection* proj;   /* the current frame's pose, camera and scale table */
+  const int32_t* rows;          /* POINTS: the local map, n_rows table rows in list order (duplicates allowed);
+                                   LAST: the table row of each keypoint of `last`, -1 for NULL or outlier */
+  int32_t n_rows;               /* POINTS only */
+  const swm_frame* last;        /* LAST only: the last frame (its octaves and angles) */
+  const int32_t* frame_rows;    /* the table row of each keypoint of tgt, -1 for none; may be NULL (none) */
+  float th;
+  float nnratio;                /* POINTS: mfNNratio of the ratio test (:110-113) */
+  int32_t check_ori;            /* LAST: mbCheckOrientation */
+  const swm_track_out* track;   /* POINTS, may be NULL */
+  int32_t* assignment;          /* tgt->n, in/out: list index (POINTS) or last-frame keypoint (LAST) at accepted slots;
+                                   with check_ori a slot assigned and then pruned comes back as -1 */
+  int32_t nmatches;             /* out */
+  int32_t n_to_match;           /* out, POINTS: rows in view (Tracking.cc:993-996) */
+} swm_localmap_job;
+/* POINTS: rows of frame_rows (bad ones excepted: SearchLocalPoints NULLs those first) are stamped as seen and skipped;
+ * bad rows are skipped; isInFrustum(pMP, 0.5) for the others in list order; a slot of tgt is unavailable when its
+ * frame row has observations and is not bad; ratio test, TH_HIGH, no orientation check.
+ * LAST: sources are the last frame's keypoints with a row; levels [octave - 1, octave + 1], the last keypoint's angle;
+ * blocks = Observations() > 0; a slot of tgt is unavailable when its frame row has observations; TH_HIGH.
+ * A batch uploads the row lists, poses and scale tables of all jobs in one copy, runs seven launches (one projection
+ * kernel, then those of swm_match_window_batch) and downloads once.  Jobs may share a table. */
+int swm_match_local_map_batch(swm_matcher* m, swm_localmap_job* jobs, int njobs);
+int swm_match_local_map(swm_matcher* m, const swm_frame* tgt, swm_mappoints* t, const swm_projection* proj,
+                        const int32_t* rows, int n_rows, const int32_t* frame_rows, float th, float nnratio,
+                        const swm_track_out* track, int32_t* assignment, int* nmatches, int* n_to_match);
+int swm_match_last_frame(swm_matcher* m, const swm_frame* cur, const swm_frame* last, swm_mappoints* t,
+                         const swm_projection* proj, const int32_t* last_rows, const int32_t* cur_rows, float th,
+                         int check_ori, int32_t* assignment, int* nmatches);
+
 /* ------------------------------------------------------------------ DBoW2 transform (SURVEY section 8(f) rank 2)
  * TemplatedVocabulary<FORB>::transform(features, BowVector&, FeatureVector&, levelsup)
  * (code/Thirdparty/DBoW2/DBoW2/TemplatedVocabulary.h:1151-1218, per feature :1242-1283) as called by

@@ -88,6 +88,26 @@ class BowJob(C.Structure):
                 ("nmatches", C.c_int32)]
 
 
+class Projection(C.Structure):
+    _fields_ = [("Tcw", C.c_float * 12), ("fx", C.c_float), ("fy", C.c_float), ("cx", C.c_float), ("cy", C.c_float),
+                ("scale_factors", C.c_void_p), ("log_scale_factor", C.c_float), ("nlevels", C.c_int32)]
+
+
+class TrackOut(C.Structure):
+    _fields_ = [("in_view", C.c_void_p), ("u", C.c_void_p), ("v", C.c_void_p), ("view_cos", C.c_void_p),
+                ("level", C.c_void_p)]
+
+
+LOCALMAP_POINTS, LOCALMAP_LAST = 0, 1
+
+
+class LocalMapJob(C.Structure):
+    _fields_ = [("mode", C.c_int32), ("tgt", C.c_void_p), ("table", C.c_void_p), ("proj", C.c_void_p),
+                ("rows", C.c_void_p), ("n_rows", C.c_int32), ("last", C.c_void_p), ("frame_rows", C.c_void_p),
+                ("th", C.c_float), ("nnratio", C.c_float), ("check_ori", C.c_int32), ("track", C.c_void_p),
+                ("assignment", C.c_void_p), ("nmatches", C.c_int32), ("n_to_match", C.c_int32)]
+
+
 # every symbol include/swm_orb.h declares: (name, restype, argtypes)
 _vp, _i, _f, _sz, _i64 = C.c_void_p, C.c_int, C.c_float, C.c_size_t, C.c_int64
 SYMBOLS = [
@@ -144,6 +164,15 @@ SYMBOLS = [
     ("swm_match_bow_batch", _i, [_vp, _vp, _i]),
     ("swm_frames_from_extractor", _i, [_vp, _i, _vp, _vp, _vp, _vp]),
     ("swm_matcher_last_device_ms", C.c_float, [_vp]),
+    ("swm_mappoints_create", _i, [_i, _i, _vp]),
+    ("swm_mappoints_destroy", None, [_vp]),
+    ("swm_mappoints_last_error", C.c_char_p, [_vp]),
+    ("swm_mappoints_size", C.c_int32, [_vp]),
+    ("swm_mappoints_upsert", _i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    ("swm_predict_scale_thresholds", _i, [_f, C.c_int32, _vp]),
+    ("swm_match_local_map_batch", _i, [_vp, _vp, _i]),
+    ("swm_match_local_map", _i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _f, _f, _vp, _vp, _vp, _vp]),
+    ("swm_match_last_frame", _i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _vp, _vp]),
     ("swm_vocab_create", _i, [_i, _vp, _sz, _vp]),
     ("swm_vocab_destroy", None, [_vp]),
     ("swm_vocab_last_error", C.c_char_p, [_vp]),

@@ -1321,6 +1321,10 @@ struct swm_matcher {
   size_t bcand_cap = 0;
   cudaEvent_t bev[2] = {nullptr, nullptr};  // around the kernels of the last batch call (swm_matcher_last_device_ms)
   float last_device_ms = 0.f;
+  // PredictScale's level thresholds of the last scale table a projection call used (swm_predict_scale_thresholds)
+  float thr_lsf = 0.f;
+  int thr_n = 0;
+  float thr[SWM_MAX_LEVELS] = {};
   // upload arena: every host array of a call is packed into one pinned buffer and sent with ONE copy
   uint8_t* h_arena = nullptr;
   uint8_t* d_arena = nullptr;
@@ -2811,4 +2815,5 @@ int frame_device_view(const swm_frame* f, FrameDeviceView* out) {
 }
 }  // namespace swm
 
+#include "mappoints.cuh"
 #include "match_batch.cuh"

@@ -284,6 +284,16 @@ namespace {
 
 using namespace swm;
 
+// A projection job (swm_match_local_map*): the caller's job, its table and the level thresholds of its scale table.
+// `wq` carries only the number of sources; lm_project_kernel writes the query rows on the device.
+struct LocalMapHost {
+  swm_localmap_job* job;
+  swm_mappoints* table;
+  swm_window_query wq;
+  float thr[SWM_MAX_LEVELS];
+  size_t off_track = 0;
+};
+
 // One matching problem as the entry points hand it over.
 struct HostJob {
   int kind = kJobWindow;
@@ -299,6 +309,7 @@ struct HostJob {
   int check_ori = 0;
   int32_t* out = nullptr;
   int32_t* nmatches = nullptr;
+  LocalMapHost* lm = nullptr;
   // filled by run_batch
   size_t off_out = 0, off_n = 0, off_prev = 0;
   int n_out = 0;
@@ -369,6 +380,66 @@ bool featvec_ok(const swm_featvec* fv) {
   return true;
 }
 
+// A projection job's device record: its operands packed into the arena, its query rows carved from the scratch (the
+// projection kernel writes them), its tracking fields pointed into the in/out region that comes back with the results.
+LocalMapDev lm_dev(swm_matcher* m, Packer& pk, Carver& cv, const LocalMapHost& h, int n2, int check_ori, size_t off_n) {
+  const swm_localmap_job& w = *h.job;
+  const size_t M = (size_t)h.wq.m;
+  LocalMapDev L;
+  memset(&L, 0, sizeof(L));
+  L.mode = w.mode;
+  L.m = (int)M;
+  L.n2 = n2;
+  L.nlevels = w.proj->nlevels;
+  L.rows = pk.put<int32_t>(w.rows, M * 4);
+  L.frame_rows = w.frame_rows ? pk.put<int32_t>(w.frame_rows, (size_t)n2 * 4) : nullptr;
+  L.nwords = (h.table->size + 31) / 32;
+  L.seen = w.mode == SWM_LOCALMAP_POINTS ? cv.take<uint32_t>((size_t)L.nwords) : nullptr;
+  L.t = h.table->view();
+  memcpy(L.T, w.proj->Tcw, sizeof(L.T));
+  L.fx = w.proj->fx; L.fy = w.proj->fy; L.cx = w.proj->cx; L.cy = w.proj->cy;
+  const FrameDev& d = w.tgt->dev;
+  L.min_x = d.min_x; L.max_x = d.max_x; L.min_y = d.min_y; L.max_y = d.max_y;
+  L.th = w.th;
+  for (int k = 0; k < L.nlevels; k++) L.sf[k] = w.proj->scale_factors[k];
+  for (int k = 0; k + 1 < L.nlevels; k++) L.thr[k] = h.thr[k];
+  if (w.mode == SWM_LOCALMAP_LAST) {
+    L.last_octave = w.last->dev.octave;
+    L.last_angle = w.last->dev.angle;
+  }
+  L.u = cv.take<float>(M); L.v = cv.take<float>(M); L.radius = cv.take<float>(M);
+  L.min_level = cv.take<int32_t>(M); L.max_level = cv.take<int32_t>(M);
+  L.valid = cv.take<uint8_t>(M); L.blocks = cv.take<uint8_t>(M);
+  L.desc = cv.take<uint4>(2 * M);
+  L.angle = check_ori ? cv.take<float>(M) : nullptr;
+  L.tgt_blocked = cv.take<uint8_t>((size_t)n2);
+  if (w.track) {
+    uint8_t* base = m->d_arena + h.off_track;
+    const size_t o1 = up256b(M), o4 = up256b(M * 4);
+    L.t_in_view = w.track->in_view ? base : nullptr;
+    L.t_u = w.track->u ? reinterpret_cast<float*>(base + o1) : nullptr;
+    L.t_v = w.track->v ? reinterpret_cast<float*>(base + o1 + o4) : nullptr;
+    L.t_cos = w.track->view_cos ? reinterpret_cast<float*>(base + o1 + 2 * o4) : nullptr;
+    L.t_level = w.track->level ? reinterpret_cast<int32_t*>(base + o1 + 3 * o4) : nullptr;
+  }
+  L.n_to_match = reinterpret_cast<int32_t*>(m->d_arena + off_n) + 2;
+  return L;
+}
+
+void lm_finish(const LocalMapHost& h, const uint8_t* down, size_t off_n) {
+  swm_localmap_job& w = *h.job;
+  w.n_to_match = reinterpret_cast<const int32_t*>(down + off_n)[2];
+  const swm_track_out* tr = w.track;
+  if (!tr) return;
+  const size_t M = (size_t)h.wq.m, o1 = up256b(M), o4 = up256b(M * 4);
+  const uint8_t* base = down + h.off_track;
+  if (tr->in_view) memcpy(tr->in_view, base, M);
+  if (tr->u) memcpy(tr->u, base + o1, M * 4);
+  if (tr->v) memcpy(tr->v, base + o1 + o4, M * 4);
+  if (tr->view_cos) memcpy(tr->view_cos, base + o1 + 2 * o4, M * 4);
+  if (tr->level) memcpy(tr->level, base + o1 + 3 * o4, M * 4);
+}
+
 // Runs the jobs that need the device (the callers have already answered the trivial ones).
 int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
   const int P = (int)jobs.size();
@@ -391,6 +462,10 @@ int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
       rows = M;
       arena += M * 58 + 10 * 256 + up256b(n2);
       scratch += 2 * up256b(M * 4);  // ev_bin, ev_tgt
+      if (j.lm) {  // rows, frame rows, tracking fields, the LocalMapDev; device-written query rows, seen stamps
+        arena += n2 * 4 + 17 * M + sizeof(LocalMapDev) + 8 * 256;
+        scratch += 58 * M + n2 + up256b((size_t)(j.lm->table->size + 31) / 32 * 4) + 12 * 256;
+      }
     } else if (j.kind == kJobInit) {
       rows = n1;
       scratch += 4 * up256b(n1 * 4) + up256b(n1) + 2 * up256b(n1 * 4);
@@ -434,8 +509,9 @@ int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
     j.off_out = pk.reserve((size_t)j.n_out * 4);
     if (j.kind == kJobWindow) memcpy(m->h_arena + j.off_out, j.out, (size_t)j.n_out * 4);
     else memset(m->h_arena + j.off_out, 0xFF, (size_t)j.n_out * 4);
-    j.off_n = pk.reserve(16);
+    j.off_n = pk.reserve(16);  // nmatches, resolve batches, n_to_match
     memset(m->h_arena + j.off_n, 0, 16);
+    if (j.lm && j.lm->job->track) j.lm->off_track = pk.reserve(17 * (size_t)j.wq->m + 5 * 256);
     if (j.kind == kJobInit) {
       j.off_prev = pk.reserve((size_t)j.f1.n() * 8);
       memcpy(m->h_arena + j.off_prev, j.prev_xy, (size_t)j.f1.n() * 8);
@@ -443,6 +519,8 @@ int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
   }
   const size_t inout_bytes = m->arena_used;
   std::vector<const swm_frame*> waits;
+  std::vector<LocalMapDev> lms;
+  std::vector<swm_mappoints*> tables;
   for (int p = 0; p < P; p++) {
     HostJob& j = jobs[p];
     BatchJob& b = bj[p];
@@ -480,18 +558,31 @@ int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
       const size_t M = (size_t)wq->m;
       b.rows_cap = wq->m;
       b.q.m = wq->m;
-      b.q.u = pk.put<float>(wq->u, M * 4);
-      b.q.v = pk.put<float>(wq->v, M * 4);
-      b.q.radius = pk.put<float>(wq->radius, M * 4);
-      b.q.min_level = pk.put<int32_t>(wq->min_level, M * 4);
-      b.q.max_level = pk.put<int32_t>(wq->max_level, M * 4);
-      b.q.valid = pk.put<uint8_t>(wq->valid, M);
-      b.q.desc = pk.put<uint4>(wq->desc, M * 32);
-      a.blocks = pk.put<uint8_t>(wq->blocks, M);
-      a.angle1 = j.check_ori ? pk.put<float>(wq->angle, M * 4) : nullptr;
-      uint8_t* blk = pk.put<uint8_t>(j.tgt_blocked, (size_t)n2);
-      if (!j.tgt_blocked && blk) memset(m->h_arena + (reinterpret_cast<uint8_t*>(blk) - m->d_arena), 0, (size_t)n2);
-      a.blocked = blk;
+      if (j.lm) {
+        lms.push_back(lm_dev(m, pk, cv, *j.lm, n2, j.check_ori, j.off_n));
+        const LocalMapDev& L = lms.back();
+        b.q.u = L.u; b.q.v = L.v; b.q.radius = L.radius;
+        b.q.min_level = L.min_level; b.q.max_level = L.max_level;
+        b.q.valid = L.valid; b.q.desc = L.desc;
+        a.blocks = L.blocks;
+        a.angle1 = L.angle;
+        a.blocked = L.tgt_blocked;
+        if (std::find(tables.begin(), tables.end(), j.lm->table) == tables.end()) tables.push_back(j.lm->table);
+        if (j.lm->job->mode == SWM_LOCALMAP_LAST) waits.push_back(j.lm->job->last);
+      } else {
+        b.q.u = pk.put<float>(wq->u, M * 4);
+        b.q.v = pk.put<float>(wq->v, M * 4);
+        b.q.radius = pk.put<float>(wq->radius, M * 4);
+        b.q.min_level = pk.put<int32_t>(wq->min_level, M * 4);
+        b.q.max_level = pk.put<int32_t>(wq->max_level, M * 4);
+        b.q.valid = pk.put<uint8_t>(wq->valid, M);
+        b.q.desc = pk.put<uint4>(wq->desc, M * 32);
+        a.blocks = pk.put<uint8_t>(wq->blocks, M);
+        a.angle1 = j.check_ori ? pk.put<float>(wq->angle, M * 4) : nullptr;
+        uint8_t* blk = pk.put<uint8_t>(j.tgt_blocked, (size_t)n2);
+        if (!j.tgt_blocked && blk) memset(m->h_arena + (reinterpret_cast<uint8_t*>(blk) - m->d_arena), 0, (size_t)n2);
+        a.blocked = blk;
+      }
       a.mode = kModeWindow;
       a.rows = wq->m;
       a.row_valid = b.q.valid;
@@ -552,8 +643,10 @@ int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
     a.row_list = cv.take<int32_t>((size_t)b.rows_cap + 64);
   }
   BatchJob* d_jobs = pk.put<BatchJob>(bj.data(), (size_t)P * sizeof(BatchJob));
+  LocalMapDev* d_lm = lms.empty() ? nullptr : pk.put<LocalMapDev>(lms.data(), lms.size() * sizeof(LocalMapDev));
   if (pk.overflow || cv.used > m->bscratch.cap) { m->err = "internal: batch arena overflow"; return SWM_E_CAPACITY; }
   for (const swm_frame* f : waits) MCK(m, cudaStreamWaitEvent(m->stream, f->ready, 0));
+  for (swm_mappoints* t : tables) MCK(m, cudaStreamWaitEvent(m->stream, t->written, 0));
   if ((rc = arena_flush(m))) return rc;
   static bool attr_set[64] = {};
   if (!attr_set[m->device & 63]) {
@@ -573,6 +666,10 @@ int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
     MCK(m, cudaMemsetAsync(job_total, 0, ((size_t)P + 1) * 4, m->stream));
     const dim3 rows_grid((unsigned)((max_rows + 7) / 8), (unsigned)P);
     MCK(m, cudaEventRecord(m->bev[0], m->stream));
+    if (d_lm) {
+      lm_project_kernel<<<(unsigned)lms.size(), kLmThreads, 0, m->stream>>>(d_lm);
+      for (swm_mappoints* t : tables) MCK(m, cudaEventRecord(t->read_done, m->stream));
+    }
     bq_prepare_kernel<<<P, 1024, 0, m->stream>>>(d_jobs, job_total, job_rows, ctl);
     bq_count_kernel<<<rows_grid, 256, 0, m->stream>>>(d_jobs);
     bq_scan_kernel<<<P, 1024, 0, m->stream>>>(d_jobs, job_total);
@@ -599,6 +696,7 @@ int run_batch(swm_matcher* m, std::vector<HostJob>& jobs) {
     memcpy(j.out, m->h_down + j.off_out, (size_t)j.n_out * 4);
     *j.nmatches = *reinterpret_cast<const int32_t*>(m->h_down + j.off_n);
     if (j.kind == kJobInit) memcpy(j.prev_xy, m->h_down + j.off_prev, (size_t)j.f1.n() * 8);
+    if (j.lm) lm_finish(*j.lm, m->h_down, j.off_n);
   }
   return SWM_OK;
 }
@@ -759,6 +857,135 @@ int swm_frames_from_extractor(swm_frame** frames, int count, swm_orb* h, const i
     FCK(f, cudaEventRecord(f->ready, v.stream));
   }
   return SWM_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------ projection from the MapPoint table
+namespace {
+
+bool rows_ok(const int32_t* r, int n, int32_t size, bool allow_none) {
+  for (int i = 0; i < n; i++)
+    if (r[i] >= size || r[i] < (allow_none ? -1 : 0)) return false;
+  return true;
+}
+
+// Validates one job and prepares its host record; a job with nothing to match is answered here (*skip = true).
+int lm_prepare(swm_matcher* m, swm_localmap_job& w, LocalMapHost& h, bool* skip) {
+  w.nmatches = 0;
+  w.n_to_match = 0;
+  *skip = true;
+  const bool last = w.mode == SWM_LOCALMAP_LAST;
+  if ((w.mode != SWM_LOCALMAP_POINTS && !last) || !w.tgt || !w.table || !w.proj || !w.assignment ||
+      (last && !w.last) || (!last && (w.n_rows < 0 || (w.n_rows > 0 && !w.rows))) || !w.proj->scale_factors ||
+      w.proj->nlevels < 1 || w.proj->nlevels > SWM_MAX_LEVELS) {
+    m->err = "bad argument in local-map job";
+    return SWM_E_INVALID;
+  }
+  for (const swm_frame* f : {w.tgt, w.last})
+    if (f && f->device != m->device) { m->err = "resident frame lives on another device"; return SWM_E_INVALID; }
+  if (w.table->device != m->device) { m->err = "MapPoint table lives on another device"; return SWM_E_INVALID; }
+  if (!w.tgt->dev.starts || (last && !w.last->dev.starts)) { m->err = "resident frame has not been built"; return SWM_E_STATE; }
+  const int M = last ? w.last->n : w.n_rows, n2 = w.tgt->n;
+  if (M > 0 && !w.rows) { m->err = "bad argument in local-map job"; return SWM_E_INVALID; }
+  const int32_t size = w.table->size;
+  if (!rows_ok(w.rows, M, size, last) || (w.frame_rows && !rows_ok(w.frame_rows, n2, size, true))) {
+    m->err = "row outside the MapPoint table";
+    return SWM_E_INVALID;
+  }
+  if (m->thr_n != w.proj->nlevels || m->thr_lsf != w.proj->log_scale_factor) {
+    if (swm_predict_scale_thresholds(w.proj->log_scale_factor, w.proj->nlevels, m->thr) != SWM_OK) {
+      m->err = "bad scale table";
+      return SWM_E_INVALID;
+    }
+    m->thr_n = w.proj->nlevels;
+    m->thr_lsf = w.proj->log_scale_factor;
+  }
+  memcpy(h.thr, m->thr, sizeof(h.thr));
+  h.job = &w;
+  h.table = w.table;
+  memset(&h.wq, 0, sizeof(h.wq));
+  h.wq.m = M;
+  *skip = M == 0 || (last && n2 == 0);
+  return SWM_OK;
+}
+
+int run_local_map(swm_matcher* m, swm_localmap_job* jobs, int njobs) {
+  if (njobs < 0 || (njobs && !jobs)) { m->err = "bad argument"; return SWM_E_INVALID; }
+  // every table the batch reads stays locked from the size check in lm_prepare until the results are back (see
+  // swm_mappoints); address order, so two batches over the same tables cannot deadlock
+  std::vector<swm_mappoints*> tables;
+  for (int p = 0; p < njobs; p++)
+    if (jobs[p].table) tables.push_back(jobs[p].table);
+  std::sort(tables.begin(), tables.end());
+  tables.erase(std::unique(tables.begin(), tables.end()), tables.end());
+  std::vector<std::unique_lock<std::mutex>> locks;
+  locks.reserve(tables.size());
+  for (swm_mappoints* t : tables) locks.emplace_back(t->mu);
+  std::vector<LocalMapHost> lh((size_t)njobs);
+  std::vector<HostJob> hj;
+  hj.reserve((size_t)njobs);
+  for (int p = 0; p < njobs; p++) {
+    swm_localmap_job& w = jobs[p];
+    bool skip;
+    int rc = lm_prepare(m, w, lh[p], &skip);
+    if (rc) return rc;
+    if (skip) continue;
+    const bool last = w.mode == SWM_LOCALMAP_LAST;
+    HostJob j;
+    j.kind = kJobWindow;
+    j.f2 = FrameSrc{nullptr, w.tgt};
+    j.wq = &lh[p].wq;
+    j.th_dist = 100;                                   // TH_HIGH, ORBmatcher.cc:111 / :1316
+    j.ratio_mode = last ? 0 : 1;
+    j.nnratio = w.nnratio;
+    j.check_ori = last ? (w.check_ori != 0) : 0;
+    j.out = w.assignment;
+    j.nmatches = &w.nmatches;
+    j.lm = &lh[p];
+    hj.push_back(j);
+  }
+  return run_batch(m, hj);
+}
+
+}  // namespace
+
+extern "C" {
+
+int swm_match_local_map_batch(swm_matcher* m, swm_localmap_job* jobs, int njobs) {
+  if (!m) return SWM_E_INVALID;
+  return run_local_map(m, jobs, njobs);
+}
+
+int swm_match_local_map(swm_matcher* m, const swm_frame* tgt, swm_mappoints* t, const swm_projection* proj,
+                        const int32_t* rows, int n_rows, const int32_t* frame_rows, float th, float nnratio,
+                        const swm_track_out* track, int32_t* assignment, int* nmatches, int* n_to_match) {
+  if (!m) return SWM_E_INVALID;
+  if (!nmatches) { m->err = "bad argument"; return SWM_E_INVALID; }
+  swm_localmap_job j;
+  memset(&j, 0, sizeof(j));
+  j.mode = SWM_LOCALMAP_POINTS;
+  j.tgt = tgt; j.table = t; j.proj = proj; j.rows = rows; j.n_rows = n_rows; j.frame_rows = frame_rows;
+  j.th = th; j.nnratio = nnratio; j.track = track; j.assignment = assignment;
+  const int rc = run_local_map(m, &j, 1);
+  *nmatches = j.nmatches;
+  if (n_to_match) *n_to_match = j.n_to_match;
+  return rc;
+}
+
+int swm_match_last_frame(swm_matcher* m, const swm_frame* cur, const swm_frame* last, swm_mappoints* t,
+                         const swm_projection* proj, const int32_t* last_rows, const int32_t* cur_rows, float th,
+                         int check_ori, int32_t* assignment, int* nmatches) {
+  if (!m) return SWM_E_INVALID;
+  if (!nmatches) { m->err = "bad argument"; return SWM_E_INVALID; }
+  swm_localmap_job j;
+  memset(&j, 0, sizeof(j));
+  j.mode = SWM_LOCALMAP_LAST;
+  j.tgt = cur; j.last = last; j.table = t; j.proj = proj; j.rows = last_rows; j.frame_rows = cur_rows;
+  j.th = th; j.check_ori = check_ori; j.assignment = assignment;
+  const int rc = run_local_map(m, &j, 1);
+  *nmatches = j.nmatches;
+  return rc;
 }
 
 }  // extern "C"

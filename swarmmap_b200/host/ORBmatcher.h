@@ -25,6 +25,7 @@
 #include "cv_shim.h"
 #endif
 #include "../../include/swm_orb.h"
+#include "MapPointTable.h"
 
 namespace ORB_SLAM2 {
 
@@ -187,6 +188,98 @@ class ORBmatcher {
     check(window_call(resident_of(F, 0), &vf, &wq, blocked.data(), TH_HIGH, 1, 0, asg.data(), &n));
     for (int j = 0; j < f.n; j++)
       if (asg[j] >= 0) F.mvpMapPoints[j] = vpMapPoints[asg[j]];             // :115
+    return n;
+  }
+
+  // ---- Tracking::SearchLocalPoints (Tracking.cc:964-1006) with the MapPoints resident in `table`: the frame's own
+  // points (bad ones NULLed, the others IncreaseVisible, mnLastFrameSeen, mbTrackInView = false), then isInFrustum(pMP,
+  // 0.5) + PredictScale and SearchByProjection(F, vpMapPoints, th) in one GPU call, then isInFrustum's writes
+  // (mbTrackInView, mTrackProjX/Y, mTrackViewCos, mnTrackScaleLevel) and IncreaseVisible in list order.  F must be
+  // resident (host/ResidentFrame.h); points the table does not hold yet are upserted first.  *nToMatch (may be NULL):
+  // the points found in view.  Monocular: mTrackProjXR is not written.
+  template <class FrameT, class MapPointT>
+  int SearchByProjection(FrameT& F, const std::vector<MapPointT*>& vpMapPoints, const float th,
+                         MapPointTable<MapPointT>& table, int* nToMatch = nullptr) {
+    const swm_frame* res = resident_of(F, 0);
+    if (!res) throw std::runtime_error("ORBmatcher::SearchByProjection(F, vpMapPoints, th, table): F must be resident");
+    for (auto& pMP : F.mvpMapPoints) {  // :970-979
+      if (!pMP) continue;
+      if (pMP->isBad()) {
+        pMP = nullptr;
+        continue;
+      }
+      pMP->IncreaseVisible();
+      pMP->mnLastFrameSeen = F.mnId;
+      pMP->mbTrackInView = false;
+    }
+    std::vector<MapPointT*> missing;
+    for (MapPointT* p : F.mvpMapPoints)
+      if (p && table.Row(p) < 0) missing.push_back(p);
+    for (MapPointT* p : vpMapPoints)
+      if (table.Row(p) < 0) missing.push_back(p);
+    table.Upsert(missing);
+    const int M = (int)vpMapPoints.size(), N = F.N;
+    std::vector<int32_t> rows(M), frame_rows(N, -1), asg(N, -1), level(M);
+    for (int i = 0; i < M; i++) rows[i] = table.Row(vpMapPoints[i]);
+    for (int j = 0; j < N; j++)
+      if (F.mvpMapPoints[j]) frame_rows[j] = table.Row(F.mvpMapPoints[j]);
+    std::vector<uint8_t> in_view(M);
+    std::vector<float> u(M), v(M), view_cos(M);
+    swm_track_out tr = {in_view.data(), u.data(), v.data(), view_cos.data(), level.data()};
+    swm_projection proj = projection(F);
+    int n = 0, ntm = 0;
+    check(swm_match_local_map(m_, res, table.get(), &proj, rows.data(), M, frame_rows.data(), th, mfNNratio, &tr,
+                              asg.data(), &n, &ntm));
+    for (int i = 0; i < M; i++) {  // :985-996, in list order
+      MapPointT* pMP = vpMapPoints[i];
+      if (pMP->mnLastFrameSeen == F.mnId || pMP->isBad()) continue;
+      pMP->mbTrackInView = in_view[i] != 0;
+      if (!in_view[i]) continue;
+      pMP->mTrackProjX = u[i];
+      pMP->mTrackProjY = v[i];
+      pMP->mTrackViewCos = view_cos[i];
+      pMP->mnTrackScaleLevel = level[i];
+      pMP->IncreaseVisible();
+    }
+    if (nToMatch) *nToMatch = ntm;
+    for (int j = 0; j < N; j++)
+      if (asg[j] >= 0) F.mvpMapPoints[j] = vpMapPoints[asg[j]];  // ORBmatcher.cc:115
+    return n;
+  }
+
+  // ---- SearchByProjection(CurrentFrame, LastFrame, th, bMono) (ORBmatcher.cc:1223-1354) with the last frame's points
+  // projected on the GPU from `table`.  Both frames must be resident; points the table does not hold yet are upserted.
+  template <class FrameT, class MapPointT>
+  int SearchByProjection(FrameT& CurrentFrame, const FrameT& LastFrame, const float th, const bool bMono,
+                         MapPointTable<MapPointT>& table) {
+    if (!bMono) throw std::runtime_error("ORBmatcher::SearchByProjection: stereo/RGB-D branch not supported (monocular SwarmMap)");
+    const swm_frame *cur = resident_of(CurrentFrame, 0), *last = resident_of(LastFrame, 0);
+    if (!cur || !last) throw std::runtime_error("ORBmatcher::SearchByProjection(cur, last, th, bMono, table): both frames must be resident");
+    std::vector<MapPointT*> missing;
+    for (int i = 0; i < LastFrame.N; i++) {
+      MapPointT* p = LastFrame.mvpMapPoints[i];
+      if (p && !LastFrame.mvbOutlier[i] && table.Row(p) < 0) missing.push_back(p);
+    }
+    for (MapPointT* p : CurrentFrame.mvpMapPoints)
+      if (p && table.Row(p) < 0) missing.push_back(p);
+    table.Upsert(missing);
+    std::vector<int32_t> last_rows(LastFrame.N, -1), cur_rows(CurrentFrame.N, -1);
+    for (int i = 0; i < LastFrame.N; i++) {  // :1247-1250
+      MapPointT* p = LastFrame.mvpMapPoints[i];
+      if (p && !LastFrame.mvbOutlier[i]) last_rows[i] = table.Row(p);
+    }
+    for (int j = 0; j < CurrentFrame.N; j++)
+      if (CurrentFrame.mvpMapPoints[j]) cur_rows[j] = table.Row(CurrentFrame.mvpMapPoints[j]);
+    const int32_t kUntouched = -3;
+    std::vector<int32_t> asg(CurrentFrame.N, kUntouched);
+    swm_projection proj = projection(CurrentFrame);
+    int n = 0;
+    check(swm_match_last_frame(m_, cur, last, table.get(), &proj, last_rows.data(), cur_rows.data(), th,
+                               mbCheckOrientation, asg.data(), &n));
+    for (int j = 0; j < CurrentFrame.N; j++) {
+      if (asg[j] >= 0) CurrentFrame.mvpMapPoints[j] = LastFrame.mvpMapPoints[asg[j]];  // :1317
+      else if (asg[j] == -1) CurrentFrame.mvpMapPoints[j] = nullptr;
+    }
     return n;
   }
 
@@ -715,6 +808,19 @@ class ORBmatcher {
       for (int c = 0; c < 3; c++) R[3 * r + c] = Tcw.template at<float>(r, c);
       t[r] = Tcw.template at<float>(r, 3);
     }
+  }
+  // The frame's pose, camera and scale table as the tracking projections take them.
+  template <class FrameT>
+  static swm_projection projection(const FrameT& F) {
+    swm_projection p;
+    std::memset(&p, 0, sizeof(p));
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 4; c++) p.Tcw[4 * r + c] = F.mTcw.template at<float>(r, c);
+    p.fx = F.fx; p.fy = F.fy; p.cx = F.cx; p.cy = F.cy;
+    p.scale_factors = F.mvScaleFactors.data();
+    p.log_scale_factor = F.mfLogScaleFactor;
+    p.nlevels = (int32_t)F.mvScaleFactors.size();
+    return p;
   }
   template <class MatT>
   static void world_pos(const MatT& p, float x[3]) { for (int i = 0; i < 3; i++) x[i] = p.template at<float>(i); }

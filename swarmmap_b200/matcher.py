@@ -10,7 +10,7 @@ import numpy as np
 from . import _lib
 from ._lib import FeatVec, FrameView, SwmError, WindowQuery, check, ptr
 
-__all__ = ["ORBmatcher", "Frame", "FeatureVector", "ResidentFrame", "Camera"]
+__all__ = ["ORBmatcher", "Frame", "FeatureVector", "ResidentFrame", "Camera", "MapPointTable"]
 
 GRID_COLS, GRID_ROWS = 64, 48
 
@@ -510,6 +510,134 @@ def _search_for_triangulation(self, KF1, fv1, no_mp1, KF2, fv2, no_mp2, F12, ex,
 
 
 ORBmatcher.SearchForTriangulation = _search_for_triangulation
+
+
+class MapPointTable:
+    """MapPoints resident on one device (world position, normal, mfMinDistance / mfMaxDistance, descriptor,
+    Observations() > 0, bad flag), one row each, for the tracking projections ORBmatcher.search_local_map /
+    search_last_frame.  Rows are the caller's: LocalMapping rewrites a point with upsert when it changes, and a query
+    uploads only row indices and the pose.  An upsert never overtakes a query still reading the table, and a query
+    sees every upsert issued before it."""
+
+    def __init__(self, device=0, capacity=0):
+        self._lib = _lib.load()
+        self._h = C.c_void_p()
+        rc = self._lib.swm_mappoints_create(int(device), int(capacity), C.byref(self._h))
+        if rc != 0:
+            msg = self._lib.swm_mappoints_last_error(None)
+            raise SwmError(f"swm_mappoints_create: {_lib.ERRORS.get(rc, rc)}: {msg.decode() if msg else ''}")
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.swm_mappoints_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def size(self):
+        return int(self._lib.swm_mappoints_size(self._h))
+
+    def upsert(self, rows, pos, normal, min_d, max_d, desc, has_obs, bad=None):
+        """Writes rows (a row given twice takes its last entry); pos / normal (n, 3), desc (n, 32)."""
+        rows = np.ascontiguousarray(rows, np.int32).reshape(-1)
+        n = len(rows)
+        a = [np.ascontiguousarray(pos, np.float32).reshape(n, 3), np.ascontiguousarray(normal, np.float32).reshape(n, 3),
+             np.ascontiguousarray(min_d, np.float32).reshape(n), np.ascontiguousarray(max_d, np.float32).reshape(n),
+             np.ascontiguousarray(desc, np.uint8).reshape(n, 32), np.ascontiguousarray(has_obs, np.uint8).reshape(n),
+             np.ascontiguousarray(np.zeros(n, np.uint8) if bad is None else bad, np.uint8).reshape(n)]
+        rc = self._lib.swm_mappoints_upsert(self._h, n, ptr(rows), *[ptr(x) for x in a])
+        if rc != 0:
+            raise SwmError(f"swm_mappoints_upsert: {_lib.ERRORS.get(rc, rc)}: "
+                           f"{self._lib.swm_mappoints_last_error(self._h).decode()}")
+        return self
+
+
+def _projection(Tcw, K, scale_factors, log_scale_factor):
+    T = np.ascontiguousarray(np.asarray(Tcw, np.float32)[:3, :4]).reshape(12)
+    sf = np.ascontiguousarray(scale_factors, np.float32)
+    p = _lib.Projection((C.c_float * 12)(*[float(x) for x in T]), *[float(np.float32(k)) for k in K], ptr(sf).value,
+                        float(np.float32(log_scale_factor)), len(sf))
+    return p, sf
+
+
+def _localmap_job(self, keep, mode, F, table, Tcw, K, log_scale_factor, rows, frame_rows=None, th=1.0, last=None,
+                  scale_factors=None, track=True, assignment=None):
+    """One swm_localmap_job.  Returns (job, outputs dict)."""
+    if not isinstance(F, ResidentFrame) or (last is not None and not isinstance(last, ResidentFrame)):
+        raise TypeError("the tracking projections take resident frames")
+    sf = F.mvScaleFactors if scale_factors is None else scale_factors
+    proj, sfa = _projection(Tcw, K, sf, log_scale_factor)
+    rows = np.ascontiguousarray(rows, np.int32).reshape(-1)
+    fr = np.ascontiguousarray(frame_rows, np.int32).reshape(-1) if frame_rows is not None else None
+    if fr is not None and len(fr) != F.N:  # the library reads one entry per keypoint
+        raise ValueError(f"frame_rows has {len(fr)} entries, the frame {F.N} keypoints")
+    if mode == _lib.LOCALMAP_LAST and (last is None or len(rows) != last.N):
+        raise ValueError("the last-frame projection takes one row per keypoint of `last`")
+    out = dict(assignment=np.full(F.N, -1 if mode == _lib.LOCALMAP_POINTS else -3, np.int32)
+               if assignment is None else assignment)
+    tr = None
+    if mode == _lib.LOCALMAP_POINTS and track:
+        m = len(rows)
+        out["track"] = dict(in_view=np.zeros(m, np.uint8), u=np.zeros(m, np.float32), v=np.zeros(m, np.float32),
+                            view_cos=np.zeros(m, np.float32), level=np.zeros(m, np.int32))
+        t = out["track"]
+        tr = _lib.TrackOut(ptr(t["in_view"]).value, ptr(t["u"]).value, ptr(t["v"]).value, ptr(t["view_cos"]).value,
+                           ptr(t["level"]).value)
+    keep.extend([proj, sfa, rows, fr, tr, out])
+    job = _lib.LocalMapJob(mode, F._h, table._h, C.addressof(proj), ptr(rows).value, len(rows),
+                           last._h if last is not None else None, ptr(fr).value if fr is not None else None, float(th),
+                           self.mfNNratio, int(self.mbCheckOrientation), C.addressof(tr) if tr is not None else None,
+                           ptr(out["assignment"]).value, 0, 0)
+    return job, out
+
+
+def _search_local_map(self, F, table, Tcw, K, log_scale_factor, rows, frame_rows=None, th=1.0, scale_factors=None,
+                      track=True):
+    """Tracking::SearchLocalPoints (Tracking.cc:964-1006) on the device: the MapPoints of the local map (table rows
+    in list order) that the current frame does not hold already and that pass isInFrustum(pMP, 0.5) are matched into
+    F with SearchByProjection(F, vpMapPoints, th).  frame_rows: the table row of each keypoint of F or -1.
+    Returns (nmatches, assignment = list index per keypoint or -1, n_to_match, tracking fields of the list or None)."""
+    r = _search_local_map_batch(self, [dict(F=F, table=table, Tcw=Tcw, K=K, log_scale_factor=log_scale_factor, rows=rows,
+                                            frame_rows=frame_rows, th=th, scale_factors=scale_factors, track=track)])
+    return r[0]
+
+
+def _search_last_frame(self, cur, last, table, Tcw, K, log_scale_factor, last_rows, cur_rows=None, th=15.0,
+                       scale_factors=None, assignment=None):
+    """SearchByProjection(cur, last, th, bMono = true), ORBmatcher.cc:1223-1354, from the table.  last_rows: the table
+    row of each keypoint of `last`, -1 for NULL or outlier.  assignment (in/out, default -3 = untouched): the
+    last-frame keypoint matched at each slot of cur, -1 where the rotation check pruned it.  Returns (nmatches,
+    assignment)."""
+    r = _search_local_map_batch(self, [dict(mode=_lib.LOCALMAP_LAST, F=cur, last=last, table=table, Tcw=Tcw, K=K,
+                                            log_scale_factor=log_scale_factor, rows=last_rows, frame_rows=cur_rows, th=th,
+                                            scale_factors=scale_factors, assignment=assignment)])
+    return r[0][0], r[0][1]
+
+
+def _search_local_map_batch(self, jobs):
+    """jobs: dicts with search_local_map's arguments (mode LOCALMAP_POINTS, the default) or search_last_frame's
+    (mode LOCALMAP_LAST, with F = cur and rows = last_rows).  One upload, seven launches, one download.
+    Returns [(nmatches, assignment, n_to_match, track-or-None)]."""
+    keep, outs = [], []
+    arr = (_lib.LocalMapJob * len(jobs))()
+    for i, kw in enumerate(jobs):
+        kw = dict(kw)
+        mode = kw.pop("mode", _lib.LOCALMAP_POINTS)
+        arr[i], out = _localmap_job(self, keep, mode, **kw)
+        outs.append(out)
+    self._check(self._lib.swm_match_local_map_batch(self._h, arr, len(jobs)), "swm_match_local_map_batch")
+    return [(int(arr[i].nmatches), outs[i]["assignment"], int(arr[i].n_to_match), outs[i].get("track"))
+            for i in range(len(jobs))]
+
+
+ORBmatcher.search_local_map = _search_local_map
+ORBmatcher.search_last_frame = _search_last_frame
+ORBmatcher.search_local_map_batch = _search_local_map_batch
 
 
 def smoke(kps, desc):
