@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 
 import ref_matcher_lib as R
+from matcher_cases import random_frame
 from swarmmap_b200 import synth
 from swarmmap_b200.matcher import FeatureVector, Frame
 
@@ -32,26 +33,6 @@ def frames(oracle):
     ex = oracle.Extractor(600, 1.2, 8, 20, 7)
     sf = oracle.scale_tables(1.2, 8)[0]
     return [Frame.from_keypoints(*ex(img), W, H, sf) for img in seq]
-
-
-def random_frame(rng, n, bits=None, bounds=(0.0, 0.0, float(W), float(H)), cluster=False):
-    """Synthetic frame: tie-heavy when `bits` is small (descriptors differ in few bits), clustered positions."""
-    if cluster:
-        c = rng.uniform([40, 40], [W - 40, H - 40], (12, 2))
-        xy = c[rng.integers(0, 12, n)] + rng.normal(0, 9, (n, 2))
-    else:
-        xy = rng.uniform([bounds[0] - 5, bounds[1] - 5], [bounds[2] + 5, bounds[3] + 5], (n, 2))
-    octave = rng.integers(0, 8, n)
-    angle = rng.uniform(0, 360, n)
-    if bits is None:
-        desc = rng.integers(0, 256, (n, 32), dtype=np.uint8)
-    else:
-        base = rng.integers(0, 256, (1, 32), dtype=np.uint8)
-        flip = np.zeros((n, 256), np.uint8)
-        for i in range(n):
-            flip[i, rng.integers(0, 256, bits)] = 1
-        desc = base ^ np.packbits(flip, axis=1)
-    return Frame(xy[:, 0], xy[:, 1], octave, angle, desc, bounds)
 
 
 # ------------------------------------------------------------------------------------------------ primitives
