@@ -566,7 +566,8 @@ float swm_kfdb_last_device_ms(const swm_kfdb* db);
 
 /* ------------------------------------------------------------------ place-recognition shard (config 5) */
 typedef struct swm_db swm_db; /* one GPU's shard of the keyframe-descriptor database */
-/* desc: ndesc x 32 bytes (host), kf_of_desc optional (NULL -> desc i belongs to kf i / desc_per_kf). */
+/* desc: ndesc x 32 bytes (host), copied to the device; descriptor i belongs to keyframe first_kf_id + i / desc_per_kf
+ * and has the global index first_kf_id * desc_per_kf + i.  swm_db_create_device takes a device array (not copied). */
 int swm_db_create(int device, const uint8_t* desc, int64_t ndesc, int32_t desc_per_kf, int64_t first_kf_id,
                   swm_db** out);
 int swm_db_create_device(int device, const uint8_t* d_desc, int64_t ndesc, int32_t desc_per_kf,
