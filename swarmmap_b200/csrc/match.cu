@@ -16,8 +16,6 @@
 // by resolve_kernel (speculative batches of 32 rows, in-order commit), which keeps match indices
 // bit-exact.  The place-recognition shard scan uses the u8 tensor-core MMA (db_top2_mma_kernel).
 #include <algorithm>
-#include <chrono>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <dlfcn.h>
@@ -369,8 +367,6 @@ struct ResolveArgs {
   int check_ori;
   // state / outputs (global memory, single warp)
   uint8_t* blocked;         // n2 (pre-initialised by the host for window mode)
-  int32_t* matched_dist;    // n2 (init mode)
-  int32_t* matches21;       // n2 (init mode)
   int32_t* out;             // init: matches12[n1]; window: assignment[n2]; bowFrame: n2; bowKf: n1
   int32_t* ev_bin;          // per source: histogram bin of its accepted match (-1 none)
   int32_t* ev_tgt;          // per source: index stored in rotHist (what gets pruned)
@@ -1313,7 +1309,7 @@ struct swm_matcher {
   DevBuf iq[5];    // SearchForInitialization's source rows, built on the device (owned)
   DevBuf rowlist;  // resolve_kernel's compacted row list
   DevBuf rows[5];  // row_count, row_start, cand_idx, cand_val, row_src
-  DevBuf state[7]; // blocked, matched_dist, matches21, out, ev_bin, ev_tgt, nmatches/prev
+  DevBuf state[5]; // blocked, out, ev_bin / best_dist, ev_tgt, nmatches
   // batch calls (match_batch.cuh): per-call scratch and the shared candidate buffers (index, level | distance),
   // grow-only, sized from earlier calls
   DevBuf bscratch;
@@ -1382,21 +1378,6 @@ struct FrameSrc {
   const swm_frame_view* host;
   const swm_frame* dev;
   int n() const { return dev ? dev->n : host->n; }
-};
-
-// SWM_MATCH_PROFILE=1: print host-side phase times of each matcher call to stderr (debug aid).
-struct PhaseTimer {
-  bool on;
-  cudaStream_t st;
-  std::chrono::steady_clock::time_point t0;
-  explicit PhaseTimer(cudaStream_t s) : on(getenv("SWM_MATCH_PROFILE") != nullptr), st(s) { t0 = std::chrono::steady_clock::now(); }
-  void mark(const char* what) {
-    if (!on) return;
-    cudaStreamSynchronize(st);
-    auto t1 = std::chrono::steady_clock::now();
-    fprintf(stderr, "[swm match] %-18s %8.1f us\n", what, std::chrono::duration<double, std::micro>(t1 - t0).count());
-    t0 = t1;
-  }
 };
 
 #define MCK(m, call)                                   \
@@ -1849,17 +1830,12 @@ int match_init_impl(swm_matcher* m, const FrameSrc& f1, const FrameSrc& f2, floa
   int total = 0;
   if ((rc = build_window_rows(m, d2, q, &total))) return rc;
   // state
-  MCK(m, m->state[1].ensure((size_t)n2 * 4));
-  MCK(m, m->state[2].ensure((size_t)n2 * 4));
+  MCK(m, m->state[1].ensure((size_t)n1 * 4));
+  MCK(m, m->state[2].ensure((size_t)n1 * 4));
   MCK(m, m->state[3].ensure((size_t)n1 * 4));
-  MCK(m, m->state[4].ensure((size_t)n1 * 4));
-  MCK(m, m->state[5].ensure((size_t)n1 * 4));
-  MCK(m, m->state[6].ensure(16));
-  std::vector<int32_t> big(n2, 0x7FFFFFFF);
-  MCK(m, cudaMemcpyAsync(m->state[1].p, big.data(), (size_t)n2 * 4, cudaMemcpyHostToDevice, m->stream));
-  MCK(m, cudaMemsetAsync(m->state[2].p, 0xFF, (size_t)n2 * 4, m->stream));
-  MCK(m, cudaMemsetAsync(m->state[3].p, 0xFF, (size_t)n1 * 4, m->stream));
-  MCK(m, cudaMemsetAsync(m->state[4].p, 0xFF, (size_t)n1 * 4, m->stream));
+  MCK(m, m->state[4].ensure(16));
+  MCK(m, cudaMemsetAsync(m->state[1].p, 0xFF, (size_t)n1 * 4, m->stream));
+  MCK(m, cudaMemsetAsync(m->state[2].p, 0xFF, (size_t)n1 * 4, m->stream));
   ResolveArgs a;
   memset(&a, 0, sizeof(a));
   a.mode = kModeInit;
@@ -1872,14 +1848,12 @@ int match_init_impl(swm_matcher* m, const FrameSrc& f1, const FrameSrc& f2, floa
   a.angle1 = d1.angle; a.angle2 = d2.angle;
   a.nnratio = nnratio;
   a.check_ori = check_ori;
-  a.matched_dist = m->state[1].as<int32_t>();
-  a.matches21 = m->state[2].as<int32_t>();
-  a.out = m->state[3].as<int32_t>();
-  a.ev_bin = m->state[4].as<int32_t>();
-  a.ev_tgt = m->state[5].as<int32_t>();
+  a.out = m->state[1].as<int32_t>();
+  a.ev_bin = m->state[2].as<int32_t>();
+  a.ev_tgt = m->state[3].as<int32_t>();
   a.prev_xy = m->q[5].as<float>();
   a.x2 = d2.x; a.y2 = d2.y;
-  a.nmatches = m->state[6].as<int32_t>();
+  a.nmatches = m->state[4].as<int32_t>();
   if ((rc = launch_resolve(m, a))) return rc;
   MCK(m, cudaGetLastError());
   if ((rc = down_begin(m, (size_t)n1 * 12 + 256))) return rc;
@@ -1895,13 +1869,31 @@ bool window_query_ok(const swm_window_query* wq, int check_ori) {
                          wq->blocks && (!check_ori || wq->angle)));
 }
 
+// Resident operands as every matcher entry point checks them: both on the matcher's device, and `built` (when not NULL)
+// holding its grid.
+int resident_ok(swm_matcher* m, const swm_frame* a, const swm_frame* b, const swm_frame* built) {
+  if (a->device != m->device || b->device != m->device) { m->err = "resident frame lives on another device"; return SWM_E_INVALID; }
+  if (built && !built->dev.starts) { m->err = "resident frame has not been built"; return SWM_E_STATE; }
+  return SWM_OK;
+}
+
+bool featvec_ok(const swm_featvec* fv) {
+  if (!fv || fv->n_nodes < 0) return false;
+  if (fv->n_nodes == 0) return true;
+  if (!fv->node_ids || !fv->offsets || !fv->feats || fv->offsets[0] < 0) return false;
+  for (int a = 0; a < fv->n_nodes; a++) {
+    if (fv->offsets[a + 1] < fv->offsets[a]) return false;
+    if (a && fv->node_ids[a] <= fv->node_ids[a - 1]) return false;  // strictly ascending node ids (std::map order)
+  }
+  return true;
+}
+
 int match_window_impl(swm_matcher* m, const FrameSrc& tgt, const swm_window_query* wq, const uint8_t* tgt_blocked,
                       int th_dist, int ratio_mode, float nnratio, int check_ori, int32_t* assignment, int* nmatches) {
   *nmatches = 0;
   const int M = wq->m, n2 = tgt.n();
   if (M == 0 || n2 == 0) return SWM_OK;
   MCK(m, cudaSetDevice(m->device));
-  PhaseTimer pt(m->stream);
   FrameDev d2;
   int rc;
   if ((rc = arena_begin(m, src_bytes(tgt) + (size_t)M * 64 + (size_t)n2 * 8 + 16 * 256))) return rc;
@@ -1919,9 +1911,8 @@ int match_window_impl(swm_matcher* m, const FrameSrc& tgt, const swm_window_quer
   std::vector<uint8_t> zero_blocked;
   if (!tgt_blocked) zero_blocked.assign((size_t)n2, 0);
   if ((rc = upload(m, m->state[0], tgt_blocked ? tgt_blocked : zero_blocked.data(), (size_t)n2))) return rc;
-  if ((rc = upload(m, m->state[3], assignment, (size_t)n2 * 4))) return rc;
+  if ((rc = upload(m, m->state[1], assignment, (size_t)n2 * 4))) return rc;
   if ((rc = arena_flush(m))) return rc;
-  pt.mark("upload (1 copy)");
   if ((rc = acquire_grid(m, 1, tgt, &d2))) return rc;
   WindowDev q;
   q.m = M;
@@ -1934,11 +1925,10 @@ int match_window_impl(swm_matcher* m, const FrameSrc& tgt, const swm_window_quer
   q.valid = m->q[4].as<uint8_t>();
   int total = 0;
   if ((rc = build_window_rows(m, d2, q, &total))) return rc;
-  pt.mark("grid + window rows");
-  MCK(m, m->state[4].ensure((size_t)M * 4));
-  MCK(m, m->state[5].ensure((size_t)M * 4));
-  MCK(m, m->state[6].ensure(16));
-  MCK(m, cudaMemsetAsync(m->state[4].p, 0xFF, (size_t)M * 4, m->stream));
+  MCK(m, m->state[2].ensure((size_t)M * 4));
+  MCK(m, m->state[3].ensure((size_t)M * 4));
+  MCK(m, m->state[4].ensure(16));
+  MCK(m, cudaMemsetAsync(m->state[2].p, 0xFF, (size_t)M * 4, m->stream));
   ResolveArgs a;
   memset(&a, 0, sizeof(a));
   a.mode = kModeWindow;
@@ -1956,24 +1946,15 @@ int match_window_impl(swm_matcher* m, const FrameSrc& tgt, const swm_window_quer
   a.nnratio = nnratio;
   a.check_ori = check_ori;
   a.blocked = m->state[0].as<uint8_t>();
-  a.out = m->state[3].as<int32_t>();
-  a.ev_bin = m->state[4].as<int32_t>();
-  a.ev_tgt = m->state[5].as<int32_t>();
-  a.nmatches = m->state[6].as<int32_t>();
-  pt.mark("state init");
+  a.out = m->state[1].as<int32_t>();
+  a.ev_bin = m->state[2].as<int32_t>();
+  a.ev_tgt = m->state[3].as<int32_t>();
+  a.nmatches = m->state[4].as<int32_t>();
   if ((rc = launch_resolve(m, a))) return rc;
-  pt.mark("resolve");
-  if (pt.on) {
-    int dbg[2] = {0, 0};
-    cudaMemcpy(dbg, a.nmatches, 8, cudaMemcpyDeviceToHost);
-    fprintf(stderr, "[swm match] rows %d batches %d matches %d\n", M, dbg[1], dbg[0]);
-  }
   if ((rc = down_begin(m, (size_t)n2 * 4 + 256))) return rc;
   if ((rc = down_copy(m, assignment, a.out, (size_t)n2 * 4))) return rc;
   if ((rc = down_copy(m, nmatches, a.nmatches, 4))) return rc;
-  if ((rc = down_finish(m))) return rc;
-  pt.mark("download");
-  return SWM_OK;
+  return down_finish(m);
 }
 
 // Merge-walk of two sorted FeatureVectors (ORBmatcher.cc:166-241, :507-581, :629-722): rows = the valid side-1
@@ -2044,13 +2025,13 @@ int match_bow_impl(swm_matcher* m, const FrameSrc& f1, const swm_featvec* fv1, c
                                                       m->rows[3].as<uint32_t>());
   MCK(m, cudaGetLastError());
   MCK(m, m->state[0].ensure((size_t)n2));
-  MCK(m, m->state[3].ensure((size_t)n_out * 4));
-  MCK(m, m->state[4].ensure((size_t)n1 * 4));
-  MCK(m, m->state[5].ensure((size_t)n1 * 4));
-  MCK(m, m->state[6].ensure(16));
+  MCK(m, m->state[1].ensure((size_t)n_out * 4));
+  MCK(m, m->state[2].ensure((size_t)n1 * 4));
+  MCK(m, m->state[3].ensure((size_t)n1 * 4));
+  MCK(m, m->state[4].ensure(16));
   MCK(m, cudaMemsetAsync(m->state[0].p, 0, (size_t)n2, m->stream));
-  MCK(m, cudaMemsetAsync(m->state[3].p, 0xFF, (size_t)n_out * 4, m->stream));
-  MCK(m, cudaMemsetAsync(m->state[4].p, 0xFF, (size_t)n1 * 4, m->stream));
+  MCK(m, cudaMemsetAsync(m->state[1].p, 0xFF, (size_t)n_out * 4, m->stream));
+  MCK(m, cudaMemsetAsync(m->state[2].p, 0xFF, (size_t)n1 * 4, m->stream));
   ResolveArgs ra;
   memset(&ra, 0, sizeof(ra));
   ra.mode = mode == 0 ? kModeBowFrame : kModeBowKf;
@@ -2065,10 +2046,10 @@ int match_bow_impl(swm_matcher* m, const FrameSrc& f1, const swm_featvec* fv1, c
   ra.nnratio = nnratio;
   ra.check_ori = check_ori;
   ra.blocked = m->state[0].as<uint8_t>();
-  ra.out = m->state[3].as<int32_t>();
-  ra.ev_bin = m->state[4].as<int32_t>();
-  ra.ev_tgt = m->state[5].as<int32_t>();
-  ra.nmatches = m->state[6].as<int32_t>();
+  ra.out = m->state[1].as<int32_t>();
+  ra.ev_bin = m->state[2].as<int32_t>();
+  ra.ev_tgt = m->state[3].as<int32_t>();
+  ra.nmatches = m->state[4].as<int32_t>();
   if ((rc = launch_resolve(m, ra))) return rc;
   MCK(m, cudaGetLastError());
   if ((rc = down_begin(m, (size_t)n_out * 4 + 256))) return rc;
@@ -2102,11 +2083,11 @@ int match_triangulation_impl(swm_matcher* m, const FrameSrc& f1, const swm_featv
   if ((rc = upload(m, m->q[0], q->scale_factors2, nl * 4))) return rc;
   if ((rc = upload(m, m->q[1], q->level_sigma2, nl * 4))) return rc;
   if ((rc = arena_flush(m))) return rc;
-  MCK(m, m->state[3].ensure((size_t)n1 * 4));
-  MCK(m, m->state[4].ensure((size_t)n1 * 4));
-  MCK(m, m->state[6].ensure(16));
-  MCK(m, cudaMemsetAsync(m->state[3].p, 0xFF, (size_t)n1 * 4, m->stream));
-  MCK(m, cudaMemsetAsync(m->state[4].p, 0xFF, (size_t)n1 * 4, m->stream));
+  MCK(m, m->state[1].ensure((size_t)n1 * 4));
+  MCK(m, m->state[2].ensure((size_t)n1 * 4));
+  MCK(m, m->state[4].ensure(16));
+  MCK(m, cudaMemsetAsync(m->state[1].p, 0xFF, (size_t)n1 * 4, m->stream));
+  MCK(m, cudaMemsetAsync(m->state[2].p, 0xFF, (size_t)n1 * 4, m->stream));
   TriDev t;
   for (int i = 0; i < 9; i++) t.F[i] = q->F12[i];
   t.ex = q->ex;
@@ -2116,14 +2097,14 @@ int match_triangulation_impl(swm_matcher* m, const FrameSrc& f1, const swm_featv
   t.nlevels = q->nlevels;
   tri_rows_kernel<<<(R + 7) / 8, 256, 0, m->stream>>>(d1, d2, m->q[4].as<uint8_t>(), R, m->rows[4].as<int32_t>(),
                                                       m->rows[1].as<int32_t>(), m->rows[2].as<int32_t>(), t, check_ori,
-                                                      m->state[3].as<int32_t>(), m->state[4].as<int32_t>());
+                                                      m->state[1].as<int32_t>(), m->state[2].as<int32_t>());
   MCK(m, cudaGetLastError());
-  tri_finalize_kernel<<<1, 1024, 0, m->stream>>>(n1, m->state[3].as<int32_t>(), m->state[4].as<int32_t>(), check_ori,
-                                                 m->state[6].as<int32_t>());
+  tri_finalize_kernel<<<1, 1024, 0, m->stream>>>(n1, m->state[1].as<int32_t>(), m->state[2].as<int32_t>(), check_ori,
+                                                 m->state[4].as<int32_t>());
   MCK(m, cudaGetLastError());
   if ((rc = down_begin(m, (size_t)n1 * 4 + 256))) return rc;
-  if ((rc = down_copy(m, matches12, m->state[3].p, (size_t)n1 * 4))) return rc;
-  if ((rc = down_copy(m, nmatches, m->state[6].p, 4))) return rc;
+  if ((rc = down_copy(m, matches12, m->state[1].p, (size_t)n1 * 4))) return rc;
+  if ((rc = down_copy(m, nmatches, m->state[4].p, 4))) return rc;
   return down_finish(m);
 }
 
@@ -2158,16 +2139,16 @@ int window_best_impl(swm_matcher* m, const FrameSrc& tgt, const swm_best_query* 
   q.valid = m->q[4].as<uint8_t>();
   int total = 0;
   if ((rc = build_window_rows(m, d2, q, &total))) return rc;
-  MCK(m, m->state[3].ensure((size_t)M * 4));
-  MCK(m, m->state[4].ensure((size_t)M * 4));
+  MCK(m, m->state[1].ensure((size_t)M * 4));
+  MCK(m, m->state[2].ensure((size_t)M * 4));
   best_rows_kernel<<<(M + 7) / 8, 256, 0, m->stream>>>(d2, M, q.u, q.v, m->rows[1].as<int32_t>(), m->rows[2].as<int32_t>(),
                                                        m->rows[3].as<uint32_t>(), gate ? m->q[9].as<float>() : nullptr,
-                                                       gate ? bq->nlevels : 0, gate ? bq->chi2 : 0.0f, m->state[3].as<int32_t>(),
-                                                       m->state[4].as<int32_t>());
+                                                       gate ? bq->nlevels : 0, gate ? bq->chi2 : 0.0f, m->state[1].as<int32_t>(),
+                                                       m->state[2].as<int32_t>());
   MCK(m, cudaGetLastError());
   if ((rc = down_begin(m, (size_t)M * 8 + 256))) return rc;
-  if ((rc = down_copy(m, best_idx, m->state[3].p, (size_t)M * 4))) return rc;
-  if ((rc = down_copy(m, best_dist, m->state[4].p, (size_t)M * 4))) return rc;
+  if ((rc = down_copy(m, best_idx, m->state[1].p, (size_t)M * 4))) return rc;
+  if ((rc = down_copy(m, best_dist, m->state[2].p, (size_t)M * 4))) return rc;
   return down_finish(m);
 }
 
@@ -2188,7 +2169,10 @@ extern "C" {
 int swm_match_init(swm_matcher* m, const swm_frame_view* f1, const swm_frame_view* f2, float* prev_xy,
                    int32_t* matches12, int window, float nnratio, int check_ori, int* nmatches) {
   if (!m) return SWM_E_INVALID;
-  if (!frame_ok(f1) || !frame_ok(f2) || !prev_xy || !matches12 || !nmatches) { m->err = "bad argument"; return SWM_E_INVALID; }
+  if (!frame_ok(f1) || !frame_ok(f2) || !prev_xy || !matches12 || !nmatches || window < 0) {
+    m->err = "bad argument";
+    return SWM_E_INVALID;
+  }
   return match_init_impl(m, FrameSrc{f1, nullptr}, FrameSrc{f2, nullptr}, prev_xy, matches12, window, nnratio, check_ori,
                          nmatches);
 }
@@ -2196,7 +2180,8 @@ int swm_match_init(swm_matcher* m, const swm_frame_view* f1, const swm_frame_vie
 int swm_match_init_resident(swm_matcher* m, const swm_frame* f1, const swm_frame* f2, float* prev_xy, int32_t* matches12,
                             int window, float nnratio, int check_ori, int* nmatches) {
   if (!m) return SWM_E_INVALID;
-  if (!f1 || !f2 || !prev_xy || !matches12 || !nmatches) { m->err = "bad argument"; return SWM_E_INVALID; }
+  if (!f1 || !f2 || !prev_xy || !matches12 || !nmatches || window < 0) { m->err = "bad argument"; return SWM_E_INVALID; }
+  if (int rc = resident_ok(m, f1, f2, f2)) return rc;
   return match_init_impl(m, FrameSrc{nullptr, f1}, FrameSrc{nullptr, f2}, prev_xy, matches12, window, nnratio, check_ori,
                          nmatches);
 }
@@ -2205,7 +2190,8 @@ int swm_match_window(swm_matcher* m, const swm_frame_view* tgt, const swm_window
                      const uint8_t* tgt_blocked, int th_dist, int ratio_mode, float nnratio, int check_ori,
                      int32_t* assignment, int* nmatches) {
   if (!m) return SWM_E_INVALID;
-  if (!frame_ok(tgt) || !window_query_ok(wq, check_ori) || !assignment || !nmatches) {
+  if (!frame_ok(tgt) || !window_query_ok(wq, check_ori) || !assignment || !nmatches ||
+      (ratio_mode != 0 && ratio_mode != 1)) {
     m->err = "bad argument";
     return SWM_E_INVALID;
   }
@@ -2217,10 +2203,11 @@ int swm_match_window_resident(swm_matcher* m, const swm_frame* tgt, const swm_wi
                               const uint8_t* tgt_blocked, int th_dist, int ratio_mode, float nnratio, int check_ori,
                               int32_t* assignment, int* nmatches) {
   if (!m) return SWM_E_INVALID;
-  if (!tgt || !window_query_ok(wq, check_ori) || !assignment || !nmatches) {
+  if (!tgt || !window_query_ok(wq, check_ori) || !assignment || !nmatches || (ratio_mode != 0 && ratio_mode != 1)) {
     m->err = "bad argument";
     return SWM_E_INVALID;
   }
+  if (int rc = resident_ok(m, tgt, tgt, tgt)) return rc;
   return match_window_impl(m, FrameSrc{nullptr, tgt}, wq, tgt_blocked, th_dist, ratio_mode, nnratio, check_ori, assignment,
                            nmatches);
 }
@@ -2229,8 +2216,8 @@ int swm_match_bow(swm_matcher* m, const swm_frame_view* f1, const swm_featvec* f
                   const swm_frame_view* f2, const swm_featvec* fv2, const uint8_t* valid2, int mode, float nnratio,
                   int check_ori, int32_t* matches, int* nmatches) {
   if (!m) return SWM_E_INVALID;
-  if (!frame_ok(f1) || !frame_ok(f2) || !fv1 || !fv2 || !valid1 || (mode == 1 && !valid2) || !matches || !nmatches ||
-      (mode != 0 && mode != 1)) {
+  if (!frame_ok(f1) || !frame_ok(f2) || !featvec_ok(fv1) || !featvec_ok(fv2) || !valid1 || (mode == 1 && !valid2) ||
+      !matches || !nmatches || (mode != 0 && mode != 1)) {
     m->err = "bad argument";
     return SWM_E_INVALID;
   }
@@ -2242,11 +2229,12 @@ int swm_match_bow_resident(swm_matcher* m, const swm_frame* f1, const swm_featve
                            const swm_frame* f2, const swm_featvec* fv2, const uint8_t* valid2, int mode, float nnratio,
                            int check_ori, int32_t* matches, int* nmatches) {
   if (!m) return SWM_E_INVALID;
-  if (!f1 || !f2 || !fv1 || !fv2 || !valid1 || (mode == 1 && !valid2) || !matches || !nmatches ||
+  if (!f1 || !f2 || !featvec_ok(fv1) || !featvec_ok(fv2) || !valid1 || (mode == 1 && !valid2) || !matches || !nmatches ||
       (mode != 0 && mode != 1)) {
     m->err = "bad argument";
     return SWM_E_INVALID;
   }
+  if (int rc = resident_ok(m, f1, f2, nullptr)) return rc;
   return match_bow_impl(m, FrameSrc{nullptr, f1}, fv1, valid1, FrameSrc{nullptr, f2}, fv2, valid2, mode, nnratio, check_ori,
                         matches, nmatches);
 }

@@ -369,17 +369,6 @@ size_t featvec_bytes(const swm_featvec* fv) {
   return up256b(nn * 4) + up256b((nn + 1) * 4) + up256b((size_t)(nn ? fv->offsets[nn] : 0) * 4) + 256;
 }
 
-bool featvec_ok(const swm_featvec* fv) {
-  if (!fv || fv->n_nodes < 0) return false;
-  if (fv->n_nodes == 0) return true;
-  if (!fv->node_ids || !fv->offsets || !fv->feats || fv->offsets[0] < 0) return false;
-  for (int a = 0; a < fv->n_nodes; a++) {
-    if (fv->offsets[a + 1] < fv->offsets[a]) return false;
-    if (a && fv->node_ids[a] <= fv->node_ids[a - 1]) return false;  // strictly ascending node ids (std::map order)
-  }
-  return true;
-}
-
 // A projection job's device record: its operands packed into the arena, its query rows carved from the scratch (the
 // projection kernel writes them), its tracking fields pointed into the in/out region that comes back with the results.
 LocalMapDev lm_dev(swm_matcher* m, Packer& pk, Carver& cv, const LocalMapHost& h, int n2, int check_ori, size_t off_n) {
@@ -720,8 +709,9 @@ int swm_match_window_batch(swm_matcher* m, swm_window_job* jobs, int njobs) {
       m->err = "bad argument in window job";
       return SWM_E_INVALID;
     }
-    if (w.tgt_resident && w.tgt_resident->device != m->device) { m->err = "resident frame lives on another device"; return SWM_E_INVALID; }
-    if (w.tgt_resident && !w.tgt_resident->dev.starts) { m->err = "resident frame has not been built"; return SWM_E_STATE; }
+    if (w.tgt_resident) {
+      if (int rc = resident_ok(m, w.tgt_resident, w.tgt_resident, w.tgt_resident)) return rc;
+    }
     w.nmatches = 0;
     HostJob j;
     j.kind = kJobWindow;
@@ -752,8 +742,9 @@ int swm_match_init_batch(swm_matcher* m, swm_init_job* jobs, int njobs) {
       m->err = "bad argument in initialization job";
       return SWM_E_INVALID;
     }
-    if (res && (w.r1->device != m->device || w.r2->device != m->device)) { m->err = "resident frame lives on another device"; return SWM_E_INVALID; }
-    if (res && !w.r2->dev.starts) { m->err = "resident frame has not been built"; return SWM_E_STATE; }
+    if (res) {
+      if (int rc = resident_ok(m, w.r1, w.r2, w.r2)) return rc;
+    }
     w.nmatches = 0;
     HostJob j;
     j.kind = kJobInit;
@@ -785,7 +776,9 @@ int swm_match_bow_batch(swm_matcher* m, swm_bow_job* jobs, int njobs) {
       m->err = "bad argument in BoW job";
       return SWM_E_INVALID;
     }
-    if (res && (w.r1->device != m->device || w.r2->device != m->device)) { m->err = "resident frame lives on another device"; return SWM_E_INVALID; }
+    if (res) {
+      if (int rc = resident_ok(m, w.r1, w.r2, nullptr)) return rc;
+    }
     w.nmatches = 0;
     HostJob j;
     j.kind = w.mode == 0 ? kJobBowFrame : kJobBowKf;
